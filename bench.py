@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one rank per GPU under torchrun for N>1)
   python bench.py --impl reference --gpus N --steps K ...   # the reference algorithm's CPU port (oracle/) on the host cores
+  python bench.py ... --dump-outputs DIR                    # also write what the last timed step computed, to compare two builds
 
 A step = one log_prob pass over one synthetic batch of the workload (default: configs[1], the CIFAR-10C-shaped conv-coupling
 specialist, onehot+vardeq, --contextflow).  Prints ONE JSON line on rank 0.
@@ -19,6 +20,7 @@ WORKLOADS = {'cfg1': 'mnist-r 1x32x32 conv generalist', 'cfg2': 'cifar10c 3x32x3
 DEFAULT_BATCH = {'cfg1': 8192, 'cfg2': 8192, 'cfg3': 1024, 'cfg4': 131072}
 REF_BATCH = {'cfg1': 256, 'cfg2': 256, 'cfg3': 64, 'cfg4': 256}          # reference default batch (config.py:10; BASELINE.md §3); cfg3: 64 (BASELINE.md §4)
 TORCH_CUDA_BATCH = {'cfg1': 2048, 'cfg2': 2048, 'cfg3': 256, 'cfg4': 8192}
+DUMP_BYTES = 64 * 10**6                                                  # --dump-outputs: all arrays of one run together
 
 
 def parse():
@@ -40,7 +42,18 @@ def parse():
     ap.add_argument('--tertiary', default='cfg3', choices=sorted(WORKLOADS) + [''], help='third workload measured in the same run: BASELINE configs[2], the ATM trans specialist ("" = none)')
     ap.add_argument('--no-parity', action='store_true', help='skip the oracle parity check of the timed batch (profiling runs)')
     ap.add_argument('--eager', action='store_true', help='launch every kernel from Python instead of replaying the captured CUDA graph')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='log_prob path of --impl ours only: after the timed steps, write the (batch, mixtures) log-probabilities the last timed '
+                         'step of each workload returned as DIR/<workload>_log_prob.npy (float32, rows in batch order; a fixed, seeded sample of '
+                         f'rows when all of them together exceed {DUMP_BYTES // 10**6} MB).  The image workloads (cfg1, cfg2) draw dequantisation '
+                         'and encoder noise from torch\'s device generator: the same build and arguments reproduce them exactly, but two builds '
+                         'that draw their noise in a different order differ by up to tens of nats per row while both are correct')
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and (a.impl != 'ours' or a.path != 'log_prob'):
+        ap.error('--dump-outputs covers the log_prob path of --impl ours only')
+    return a
 
 
 class ClockSampler(threading.Thread):
@@ -110,8 +123,8 @@ class ClockSampler(threading.Thread):
 
 
 def _reference_forward(workload, device):
-    """(log_prob(x, ctx) callable, kind, description): the UNMODIFIED reference when a complete checkout is found (baseline/_ref, made by
-    tools/install_reference.py, or /root/reference) -- its own create_model / FlowSequential.log_prob over its own torch layers --
+    """(log_prob(x, ctx) callable, kind, description): the UNMODIFIED reference when a complete checkout is found ($CFPP_REFERENCE, or
+    baseline/_ref made by tools/install_reference.py) -- its own create_model / FlowSequential.log_prob over its own torch layers --
     else the oracle port (oracle/flow_oracle.py: the same torch op sequence, pinned to the reference by tests/golden)."""
     import torch
     from contextflow_b200 import builder, synth
@@ -265,12 +278,14 @@ def measure(a, workload, B, rank, world, dev, with_e2e=True, parity=True):
     t_begin = time.perf_counter()
     ev0.record()
     for i in range(a.steps):
-        step(i)
+        out = step(i)
     ev1.record()
     barrier()
     t_end = time.perf_counter()
     if prof_range:
         torch.cuda.profiler.stop()
+    # a graph replay returns its static output buffer, which the passes below overwrite: copy the last timed step's result out now
+    last_out = out.float().cpu() if a.dump_outputs and rank == 0 else None
     ms = ev0.elapsed_time(ev1)
     launches = _cabi.launch_count() - l0 if graphed is None else graphed.launches_per_replay(*devb[0]) * a.steps
     # per-kernel durations: the same steps launched eagerly with a CUDA-event pair around every libcfpp launch (events cannot be
@@ -420,7 +435,21 @@ def measure(a, workload, B, rank, world, dev, with_e2e=True, parity=True):
                           'timed region; the timed step runs the coupling transform inside the conditioner kernel'}
     return {'value': world * B * a.steps / (ms / 1e3), 'ms_per_step': ms / a.steps, 'config': config_line(workload, B, world, conf, graphed is not None),
             'clocks': clocks, 'gpu_launches': launches, 'e2e': e2e, 'roofline': roof, 'roofline_coupling': roof_c, 'roofline_hbm_path': roof_hbm,
-            'kernels': kernels, 'parity_at_bench_batch': par}
+            'kernels': kernels, 'parity_at_bench_batch': par, 'outputs': {f'{workload}_log_prob': last_out}}
+
+
+def dump_outputs(path, arrays):
+    """Write each (rows, M) array as path/<name>.npy in float32.  When all of them together exceed DUMP_BYTES, each keeps the same share
+    of its rows: a sorted sample drawn with a fixed seed, so that two runs with the same arguments write the same rows."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    total = sum(v.numel() * 4 for v in arrays.values())
+    for name, v in arrays.items():
+        v = v.numpy().astype(np.float32)
+        if total > DUMP_BYTES:
+            keep = max(1, v.shape[0] * DUMP_BYTES // total)
+            v = v[np.sort(np.random.default_rng(0).choice(v.shape[0], keep, replace=False))]
+        np.save(os.path.join(path, f'{name}.npy'), v)
 
 
 def main():
@@ -486,6 +515,8 @@ def main():
         os.dup2(saved_stdout, 1)
         os.close(saved_stdout)
     if rank == 0:
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, {k: v for r in (res, sec, ter) if r is not None for k, v in r['outputs'].items()})
         line = {'metric': METRIC, 'value': res['value'], 'unit': UNIT, 'n_gpus': world, 'steps': a.steps, 'warmup': max(a.warmup, 3),
                 'ms_per_step': res['ms_per_step'], 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic',
                 'config': res['config'], 'clocks': res['clocks'], 'gpu_launches': res['gpu_launches'], 'e2e': res['e2e'],

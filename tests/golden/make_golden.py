@@ -1,6 +1,6 @@
-"""Generate tests/golden/*.npz by executing the UNMODIFIED reference (/root/reference) on CPU.
+"""Generate tests/golden/*.npz by executing the UNMODIFIED reference on CPU.
 
-Run in the build container only:   python tests/golden/make_golden.py
+    CFPP_REFERENCE=<upstream checkout>/contextflow python tests/golden/make_golden.py
 The reference is imported through the shim of SURVEY App. B (no reference file is edited or copied).
 Weights are overwritten with contextflow_b200.synth.fill_state (hash-derived, portable), inputs come
 from synth.make_inputs, and the reference's own torch.rand/torch.randn calls are served from a
@@ -16,10 +16,12 @@ sys.path.insert(0, ROOT)
 from contextflow_b200 import synth  # noqa: E402
 from tests.golden.cases import CASES  # noqa: E402
 
-REF = '/root/reference/contextflow'
+REF = os.environ.get('CFPP_REFERENCE', '')
 
 
 def import_reference():
+    if not os.path.isfile(os.path.join(REF, 'model.py')):
+        sys.exit('set CFPP_REFERENCE to the upstream contextflow package directory')
     sys.dont_write_bytecode = True
     sys.path.insert(0, REF)
     pkg = types.ModuleType('datasets'); pkg.__path__ = [REF + '/datasets']; pkg.corrupt = None

@@ -1,6 +1,7 @@
 """Generate tests/golden/extras.npz by executing the UNMODIFIED reference classes that create_model never builds but that can be
 constructed directly: the standalone Sigmoid / Softplus flow layers (layers/activations.py:228-264) and StudentMixtureDistribution
-(layers/distributions/student.py:44-111).  Run in the build container only:   python tests/golden/make_golden_extras.py"""
+(layers/distributions/student.py:44-111).
+    CFPP_REFERENCE=<upstream checkout>/contextflow python tests/golden/make_golden_extras.py"""
 import os, sys
 import numpy as np
 import torch

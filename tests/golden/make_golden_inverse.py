@@ -1,6 +1,6 @@
-"""Generate tests/golden/inv_*.npz and score_*.npz by executing the UNMODIFIED reference (/root/reference) on CPU.
+"""Generate tests/golden/inv_*.npz and score_*.npz by executing the UNMODIFIED reference on CPU.
 
-Run in the build container only:   python tests/golden/make_golden_inverse.py
+    CFPP_REFERENCE=<upstream checkout>/contextflow python tests/golden/make_golden_inverse.py
 Inverse direction (SURVEY §8f-3).  Two kinds of fixture:
   * full chain (models whose every layer has an executable .reverse in the reference: generalists without split priors):
     the latent z of the forward golden is pushed through `module.reverse` from the last layer to the first, exactly the loop

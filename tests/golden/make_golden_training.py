@@ -1,6 +1,6 @@
-"""Generate tests/golden/train_*.npz by executing the UNMODIFIED reference (/root/reference) on CPU with torch autograd.
+"""Generate tests/golden/train_*.npz by executing the UNMODIFIED reference on CPU with torch autograd.
 
-Run in the build container only:   python tests/golden/make_golden_training.py
+    CFPP_REFERENCE=<upstream checkout>/contextflow python tests/golden/make_golden_training.py
 Training direction (SURVEY §8f-1).  For each case the reference model (hash-derived weights, inputs and noise, as in make_golden.py)
 evaluates the training loss exactly as experiment_ad.py:204-209 writes it and calls .backward(); stored: the loss terms and the
 gradient of every trainable parameter (full tensor up to 2048 elements, else (sum, sum|.|) and the first 512 values), plus the

@@ -1,13 +1,16 @@
-"""Drop-in boundary, checked in the build container (skipped where /root/reference is absent, e.g. the GPU box):
-the reference's own, unmodified model.create_model / ContextEncoder, executed over THIS package's `layers` namespace,
-must construct, and must yield exactly the module tree / state_dict of (a) the reference over its own layers (the golden
-`keys` tables) and (b) contextflow_b200.builder.create_model, which the GPU tests and bench use in its place."""
+"""Drop-in boundary on the CPU.  Without the reference: contextflow_b200.builder.create_model, which the GPU tests and bench use, yields
+the state_dict table and layer sequence the unmodified reference recorded over its own layers (tests/golden).  With a reference checkout
+($CFPP_REFERENCE or baseline/_ref, see tools/refshim.py; skipped otherwise): the reference's own, unmodified model.create_model /
+ContextEncoder, executed over THIS package's `layers` namespace, must construct, and must yield exactly the module tree / state_dict of
+(a) the reference over its own layers (the golden `keys` tables) and (b) contextflow_b200.builder.create_model."""
 import argparse, json, os, subprocess, sys, textwrap
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = '/root/reference/contextflow'
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason='reference checkout not present')
+sys.path.insert(0, os.path.join(ROOT, 'tools'))
+import refshim  # noqa: E402
+
+REF = refshim.find_reference()
 
 SCRIPT = textwrap.dedent('''
     import sys, types, json, argparse
@@ -44,6 +47,19 @@ SCRIPT = textwrap.dedent('''
 ''')
 
 
+def test_builder_matches_reference_tables():
+    from contextflow_b200 import builder
+    from tests.golden.cases import CASES
+    from tests.helpers import load_golden
+    for name, case in CASES.items():
+        g = load_golden(name)
+        model = builder.build_named(case['conf'])
+        keys = {k: list(v.shape) for k, v in model.state_dict().items()}
+        assert keys == g['keys'] and list(keys) == list(g['keys']), f'{name}: state_dict differs from the reference over its own layers'
+        assert [type(m).__name__ for m in model.sequence_modules] == g['layer_types'], f'{name}: layer sequence differs'
+
+
+@pytest.mark.skipif(REF is None, reason='no checkout of the unmodified reference (CFPP_REFERENCE)')
 def test_reference_create_model_runs_over_replacement_layers():
     from tests.golden.cases import CASES
     from tests.helpers import load_golden

@@ -1,8 +1,8 @@
 """The drop-in boundary end to end on the GPU (SURVEY §8b; VERDICT r1 next-7): the reference's UNMODIFIED experiment loops
 (experiment_ad.py:184-291, experiment_cl.py:107-215: eval_epoch, train_epoch with the AdamW model.py:289 builds, save / load of a
 generalist checkpoint into a specialist with strict=False) run over this repo's layers and over the reference's own torch layers on
-the same GPU; every reported number must agree.  Needs a complete reference checkout (baseline/_ref made by
-tools/install_reference.py, or /root/reference): skipped otherwise."""
+the same GPU; every reported number must agree.  Needs a complete reference checkout ($CFPP_REFERENCE, or baseline/_ref made by
+tools/install_reference.py): skipped otherwise."""
 import json
 import os
 import subprocess
@@ -14,7 +14,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, 'tools'))
 import refshim  # noqa: E402
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(refshim.find_reference() is None, reason='no complete reference checkout (baseline/_ref)')]
+pytestmark = [pytest.mark.gpu, pytest.mark.skipif(refshim.find_reference() is None, reason='no complete reference checkout ($CFPP_REFERENCE or baseline/_ref)')]
 
 
 def _arm(arm, kind, tmp_path):

@@ -1,4 +1,4 @@
-"""Single-process N-GPU log_prob (contextflow_b200/multigpu.py): needs at least two visible GPUs (gpurun --gpus 2); skipped otherwise."""
+"""Single-process N-GPU log_prob (contextflow_b200/multigpu.py): needs at least two visible GPUs; skipped otherwise."""
 import pytest
 import torch
 

@@ -61,9 +61,25 @@ def test_fused_plan_is_not_used_on_cpu_tensors():
             model.log_prob(x, ctx)
 
 
+def test_dump_outputs_samples_the_same_rows_within_budget(tmp_path, monkeypatch):
+    import numpy as np
+    import bench
+    monkeypatch.setattr(bench, 'DUMP_BYTES', 4000)
+    big, small = torch.arange(3000.0).reshape(1500, 2), torch.ones(10, 1)          # 12040 bytes together
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), {'big': big, 'small': small})
+    a, b = np.load(tmp_path / 'a' / 'big.npy'), np.load(tmp_path / 'b' / 'big.npy')
+    s = np.load(tmp_path / 'a' / 'small.npy')
+    assert a.dtype == s.dtype == np.float32 and np.array_equal(a, b)
+    assert a.nbytes + s.nbytes <= 4000 and a.shape[1] == 2 and s.shape == (3, 1)
+    assert np.all(np.diff(a[:, 0]) > 0) and np.all(a[:, 1] == a[:, 0] + 1)        # whole rows, in batch order
+    bench.dump_outputs(str(tmp_path / 'c'), {'small': small})                        # under the budget: every row
+    assert np.array_equal(np.load(tmp_path / 'c' / 'small.npy'), small.numpy())
+
+
 @pytest.mark.parametrize('force_port', ['1', '0'])
 def test_reference_arm_prints_one_json_line(force_port):
-    """--impl reference: the unmodified reference when a complete checkout exists (baseline/_ref or /root/reference), else the port."""
+    """--impl reference: the unmodified reference when a complete checkout exists ($CFPP_REFERENCE or baseline/_ref), else the port."""
     out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--impl', 'reference', '--workload', 'cfg4', '--batch', '64',
                           '--steps', '1', '--warmup', '1'], capture_output=True, text=True, timeout=300, cwd=ROOT,
                          env=dict(os.environ, CFPP_BENCH_FORCE_PORT=force_port))

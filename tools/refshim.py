@@ -1,8 +1,8 @@
 """Locating and importing the UNMODIFIED reference (gudovskiy/contextflow) for baselines and boundary tests.  Measurement / test
 infrastructure only: nothing under contextflow_b200/ imports this.
 
-Search order: $CFPP_REFERENCE, <repo>/baseline/_ref/contextflow (the offline install made by tools/install_reference.py: git-ignored,
-travels to the GPU box), /root/reference/contextflow (build container only).  A directory counts only when it holds the whole package
+Search order: $CFPP_REFERENCE (the `contextflow` package directory of an upstream checkout), <repo>/baseline/_ref/contextflow (the
+offline install made by tools/install_reference.py, git-ignored).  A directory counts only when it holds the whole package
 (`model.py` AND `layers/`): the reference's setup.py lists `packages=['contextflow']` without sub-packages, so a bare pip install
 lacks layers/, utils/ and datasets/ and cannot run.
 
@@ -15,7 +15,7 @@ import sys
 import types
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CANDIDATES = [os.environ.get('CFPP_REFERENCE'), os.path.join(ROOT, 'baseline', '_ref', 'contextflow'), '/root/reference/contextflow']
+CANDIDATES = [os.environ.get('CFPP_REFERENCE'), os.path.join(ROOT, 'baseline', '_ref', 'contextflow')]
 
 
 def find_reference():
