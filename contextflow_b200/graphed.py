@@ -197,12 +197,16 @@ class GraphedTrainStep:
         for p in params:
             p.grad = None                                # the captured backward allocates the static .grad tensors in the graph's pool
         self.graph = torch.cuda.CUDAGraph()
+        from . import rng
         from .layers.flowlayer import live_capture
         # live_capture: everything derived from a trainable parameter (log|det NN|, NN^-1, mixture tables, masked weights) is recomputed by
         # kernels recorded in the graph instead of being served from the version-keyed host caches the warm-up filled
+        del rng._capture_host_draws[:]
         with live_capture(), torch.cuda.graph(self.graph):
             self.loss = loss_fn(model, *self.static)
             self.loss.backward()
+        self.host_draws = list(rng._capture_host_draws)      # rng 'host' mode: device buffers that stand in for the CPU-generator draws
+        del rng._capture_host_draws[:]
 
     def attach_optimizer(self, opt):
         """Capture `opt.step()` (contextflow_b200.optim.FusedAdamW: one multi-tensor kernel, step counter and bias corrections on the
@@ -211,9 +215,9 @@ class GraphedTrainStep:
         from .optim import FusedAdamW
         if not isinstance(opt, FusedAdamW):
             raise TypeError('attach_optimizer needs a contextflow_b200.optim.FusedAdamW (a plain torch.optim.AdamW is not capturable)')
-        for gi, group in enumerate(opt.param_groups):
-            opt._plan(gi, group)                           # pointer tables and state buffers are built eagerly (host -> device copies)
+        plans = [opt._plan(gi, group) for gi, group in enumerate(opt.param_groups)]   # pointer tables and state buffers are built eagerly
         self.opt = opt
+        self.opt_params = [p for plan in plans if plan is not None for p in plan['params']]
         self.opt_graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.opt_graph):
             opt.step()
@@ -223,6 +227,7 @@ class GraphedTrainStep:
         """Optimizer update from the gradients of the last replay (after an optional gradient all-reduce)."""
         self.opt.sync_learning_rate()
         self.opt_graph.replay()
+        torch.autograd.graph.increment_version(self.opt_params)    # the replay wrote the parameters: invalidate what is cached on them
 
     def __call__(self, x, ctx, gt=None):
         self.static[0].copy_(x, non_blocking=True)
@@ -230,5 +235,7 @@ class GraphedTrainStep:
             self.static[1].copy_(ctx, non_blocking=True)
         if gt is not None:
             self.static[2].copy_(gt, non_blocking=True)
+        for buf in self.host_draws:                            # same CPU-generator stream as an eager step (uniform.py:32)
+            buf.copy_(torch.rand(buf.shape, dtype=buf.dtype))
         self.graph.replay()
         return self.loss

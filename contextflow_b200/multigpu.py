@@ -25,7 +25,7 @@ class ReplicatedLogProb:
         self.min_rows = int(min_rows)
         self._devices = devices
         self._replicas = {}            # device index -> replica of the model
-        self._sig = None
+        self._sigs = {}                # device index -> source signature the replica was last refreshed at
         self._tensors = None
         self._all_initialized = False
         self._streams = {}
@@ -54,21 +54,22 @@ class ReplicatedLogProb:
         return r
 
     def _sync(self, devs):
-        """Replicas follow the source model: parameters / buffers are re-copied whenever a version counter moved (optimizer step,
-        load_state_dict, ActNorm initialisation)."""
+        """Replicas follow the source model: a replica's parameters / buffers are re-copied whenever a version counter moved (optimizer
+        step, load_state_dict, ActNorm initialisation) since that replica was last refreshed.  Each replica keeps its own signature: a
+        call that uses fewer devices than an earlier one leaves the others alone, and a later call on them must still refresh them."""
         sig = self._signature()
-        fresh = [d for d in devs if d.index not in self._replicas]
-        reps = [self._replica(d) for d in devs]
-        if sig != self._sig:
-            src = list(self.model.parameters()) + list(self.model.buffers())
-            with torch.no_grad():
-                for d, r in zip(devs, reps):
-                    if d in fresh:
-                        continue                       # a deepcopy made just now already holds the current values
-                    dst = list(r.parameters()) + list(r.buffers())
-                    for a, b in zip(dst, src):
+        reps, src = [], None
+        for d in devs:
+            fresh = d.index not in self._replicas          # a deepcopy made just now already holds the current values
+            r = self._replica(d)
+            if not fresh and self._sigs.get(d.index) != sig:
+                if src is None:
+                    src = list(self.model.parameters()) + list(self.model.buffers())
+                with torch.no_grad():
+                    for a, b in zip(list(r.parameters()) + list(r.buffers()), src):
                         a.copy_(b, non_blocking=True)
-            self._sig = sig
+            self._sigs[d.index] = sig
+            reps.append(r)
         return reps
 
     def _initialized(self):
@@ -89,6 +90,10 @@ class ReplicatedLogProb:
         if n < 2 or not self._initialized():
             return model._log_prob_single(x, ctx)
         devs = devs[:n]
+        # a peer copy moves one dense block: row slices of a contiguous batch are contiguous.  Made here, on the caller's stream before
+        # `ready`, so that every slice's stream is ordered after it; the copies stay alive until the caller's stream has waited for all slices
+        x = x.contiguous()
+        ctx = None if ctx is None else ctx.contiguous()
         reps = self._sync(devs[1:])
         ready = torch.cuda.Event()
         cur = torch.cuda.current_stream(primary)

@@ -78,6 +78,10 @@ class FusedAdamW(_TorchAdamW):
                                                  _cabi.vp(plan['state'].data_ptr()), _cabi.vp(plan['lr'].data_ptr()), float(b1), float(b2),
                                                  float(group['eps']), float(group['weight_decay']), _cabi.vp(torch.cuda.current_stream(dev).cuda_stream))
             _cabi.check(rc, 'adamw_step')
+            if not capturing:
+                # the kernel writes through raw pointers: bump the version counters so that every value cached on them (log|det NN|,
+                # NN^-1, mixture tables, packed weights, captured log_prob graphs, multi-GPU replicas) is rebuilt
+                torch.autograd.graph.increment_version(plan['params'])
         return loss
 
     def sync_learning_rate(self):

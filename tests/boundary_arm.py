@@ -4,7 +4,7 @@
 
 Drives the reference's UNMODIFIED `AdExperiment` / `ClExperiment` (experiment_ad.py / experiment_cl.py) -- eval_epoch, train_epoch,
 save(), load() of a generalist checkpoint into a specialist (experiment_ad.py:304-323) -- over either this repo's layers
-(`replacement`: contextflow_b200.run.install_layers + CUDA graphs for inference, exactly what `python -m contextflow_b200.run
+(`replacement`: contextflow_b200.run.install_layers + the fused AdamW + CUDA graphs for inference, exactly what `python -m contextflow_b200.run
 model.py` sets up) or the reference's own torch layers (`reference`, TF32 off) on the same GPU, with identical weights
 (synth.fill_state), identical in-memory loaders and identical generator seeds.  With CFPP_RNG=reference both arms consume
 torch's generators identically, so every number they print must agree within the fp32 parity gates."""
@@ -33,6 +33,9 @@ def main(arm, kind, out_path):
     if arm == 'replacement':
         import contextflow_b200.layers as L
         assert M.FlowSequential is L.FlowSequential, 'model.py did not pick up the replacement layers'
+        if os.environ.get('CFPP_FUSED_ADAMW', '1') != '0':      # what run.py installs: optim.AdamW (model.py:289) builds the fused optimizer
+            from contextflow_b200 import optim as _optim
+            _optim.install()
     dev = torch.device(os.environ.get('CFPP_BND_DEVICE', 'cuda:0'))
     if kind == 'ad':
         from experiment_ad import AdExperiment as Exp
