@@ -13,9 +13,13 @@ in the eager warm-up), no host memory copies inside the library, every buffer al
 """
 from __future__ import annotations
 
-import torch
-
+import contextlib
+import gc
 import operator
+import weakref
+
+import torch
+from torch._utils import _flatten_dense_tensors, _unflatten_dense_tensors
 
 from . import _cabi
 
@@ -173,6 +177,212 @@ class GraphedLogProb:
         return outs
 
 
+_requires_grad_of = operator.attrgetter('requires_grad')
+_suspended = 0          # > 0 while GraphedTrainStep warms up over a model: its log_prob calls under autograd then stay eager
+
+
+@contextlib.contextmanager
+def eager_training():
+    """Calls of log_prob under autograd launch eagerly inside this block, whatever GraphedTrainLogProb is enabled."""
+    global _suspended
+    _suspended += 1
+    try:
+        yield
+    finally:
+        _suspended -= 1
+
+
+@contextlib.contextmanager
+def _leaf_aliases(model, params):
+    """While a training entry warms up and captures, every trainable parameter of `model` is replaced by a fresh leaf over the same
+    storage; yields those leaves.  The graphs read and the optimizer writes the same memory, but the capture never reaches the
+    parameters' own AccumulateGrad nodes: the caller's previous step may keep them alive, bound to the stream of an eager call, and
+    an autograd backward that synchronises with another stream cannot be captured."""
+    leaves = {id(p): torch.nn.Parameter(p.detach()) for p in params}
+    saved = [(m, k, v) for m in model.modules() for k, v in m._parameters.items() if v is not None and id(v) in leaves]
+    for m, k, v in saved:
+        m._parameters[k] = leaves[id(v)]
+    try:
+        yield [leaves[id(p)] for p in params]
+    finally:
+        for m, k, v in saved:
+            m._parameters[k] = v
+
+
+class _TrainEntry:
+    __slots__ = ('fwd', 'bwd', 'x', 'ctx', 'out', 'dlogp', 'flat', 'used', 'slots', 'params', 'frozen', 'versions', 'host_draws',
+                 'device', 'generation', 'waiting')
+
+
+class _ReplayTrain(torch.autograd.Function):
+    """Joins an entry's forward and backward graphs to the caller's autograd graph.  The trainable parameters are the inputs, so the
+    backward hands autograd one gradient per parameter and the caller's loss, backward() and optimizer stay where they are."""
+
+    @staticmethod
+    def forward(ctx, e, x, c, *params):
+        e.x.copy_(x, non_blocking=True)
+        if c is not None:
+            e.ctx.copy_(c, non_blocking=True)
+        for buf in e.host_draws:                                # rng 'host' mode: the CPU-generator draws of this forward
+            buf.copy_(torch.rand(buf.shape, dtype=buf.dtype))
+        if e.device.index != torch.cuda.current_device():
+            with torch.cuda.device(e.device):
+                e.fwd.replay()
+        else:
+            e.fwd.replay()
+        e.generation += 1
+        ctx.entry, ctx.generation = e, e.generation
+        e.waiting = weakref.ref(ctx)                            # this replay's activations wait for its backward
+        return e.out.detach().clone()                           # the caller may edit its log-probabilities in place
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, dlogp):
+        e = ctx.entry
+        if ctx.generation != e.generation:
+            raise RuntimeError('log_prob was replayed from its CUDA graph again before this backward ran, which overwrote the activations '
+                               'this backward needs.  Call backward() before the next log_prob of the same shape, or disable training '
+                               'graphs with model.enable_cuda_graphs(training=False).')
+        e.dlogp.copy_(dlogp)
+        e.bwd.replay()
+        e.waiting = None
+        # one device copy of all gradients; AccumulateGrad adopts the views as .grad without copying them again
+        views = _unflatten_dense_tensors(e.flat.clone(), e.used) if e.used else ()
+        grads = [None] * (3 + len(e.params))
+        for slot, g in zip(e.slots, views):
+            grads[3 + slot] = g
+        return tuple(grads)
+
+
+class GraphedTrainLogProb:
+    """CUDA-graph replay of `log_prob` under autograd, for a training loop that keeps its own loss, backward() and optimizer step.
+
+    Per input shape an entry holds two graphs over static buffers: the forward (log_prob_eager under autograd, derived weights
+    recomputed inside the graph: live_capture) and the backward (torch.autograd.grad of the captured log-probabilities with respect to
+    the trainable parameters, written into one flat gradient buffer).  `_ReplayTrain` joins them to the caller's autograd graph.
+
+    The first call at a key (input shapes and dtypes, model.training, which parameters require grad) runs eagerly; that call also
+    performs one-time work such as ActNorm's first-batch initialisation.  The second call captures and replays.  An entry stays valid
+    while no parameter or buffer has moved and no tensor that does not require grad has been written: trainable parameters are read
+    live by the graphs, so optimizer steps keep it valid, while values derived from frozen tensors are cached under their versions and a
+    load_state_dict forces a new eager call and capture.  MAX_ENTRIES entries are kept (e.g. the full batch and the ragged last batch),
+    the oldest is dropped first."""
+
+    MAX_ENTRIES = 2
+
+    def __init__(self, model, warmup: int = 1):
+        self.model, self.warmup = model, max(1, warmup)
+        self._entries = {}
+        self._seen = {}             # key -> state signature after the eager call at that key
+        self._tensors = None
+
+    def invalidate(self):
+        self._tensors = None
+        self._entries.clear()
+        self._seen.clear()
+
+    def _state(self):
+        ts = self._tensors
+        if ts is None:
+            self._params = list(self.model.parameters())
+            ts = self._tensors = self._params + list(self.model.buffers())
+            self._ptrs = hash(tuple(t.data_ptr() for t in ts))
+        return ts
+
+    def _signature(self, frozen):
+        return hash(tuple(map(_version_of, frozen))) ^ self._ptrs
+
+    def __call__(self, x, ctx=None):
+        if (_suspended or x.requires_grad or (ctx is not None and (ctx.requires_grad or not ctx.is_cuda))
+                or torch.cuda.is_current_stream_capturing()):
+            return self.model.log_prob_eager(x, ctx)
+        from . import rng
+        if rng._source is not None or rng._recorder is not None:   # replayed noise tapes / draw recording are host-driven
+            return self.model.log_prob_eager(x, ctx)
+        ts = self._state()
+        rg = tuple(map(_requires_grad_of, self._params))
+        key = (tuple(x.shape), x.dtype, x.device, None if ctx is None else (tuple(ctx.shape), ctx.dtype), self.model.training, rg)
+        e = self._entries.get(key)
+        if e is not None and self._signature(e.frozen) != e.versions:
+            del self._entries[key]                              # weights loaded or moved: eager once more, then a new capture
+            e = None
+        if e is None:
+            frozen = [t for t in ts if not t.requires_grad]
+            params = [p for p in self._params if p.requires_grad]
+            if (not params or any(p._backward_hooks or p._post_accumulate_grad_hooks for p in params)
+                    or self._seen.get(key) != self._signature(frozen)):
+                out = self.model.log_prob_eager(x, ctx)
+                self._seen.pop(key, None)
+                self._seen[key] = self._signature(frozen)
+                while len(self._seen) > 4 * self.MAX_ENTRIES:
+                    del self._seen[next(iter(self._seen))]
+                return out
+            e = self._capture(x, ctx, params, frozen)
+            self._entries[key] = e
+            while len(self._entries) > self.MAX_ENTRIES:
+                del self._entries[next(iter(self._entries))]
+        elif (e.waiting is not None and e.waiting() is not None) or any(p._backward_hooks or p._post_accumulate_grad_hooks for p in e.params):
+            return self.model.log_prob_eager(x, ctx)           # a replay's backward is still due, or a hook must see the eager backward
+        return _ReplayTrain.apply(e, x, ctx, *e.params)
+
+    def _capture(self, x, ctx, params, frozen):
+        # no garbage collection while the graphs are captured: a collected module tree may destroy CUDA graphs of its own, and those
+        # calls invalidate a capture in progress (torch.cuda.graph collects once before it begins, not during)
+        gc_was_enabled = gc.isenabled()
+        gc.collect()
+        gc.disable()
+        try:
+            with torch.cuda.device(x.device):
+                return self._capture_on(x, ctx, params, frozen, x.device)
+        finally:
+            if gc_was_enabled:
+                gc.enable()
+
+    def _capture_on(self, x, ctx, params, frozen, device):
+        from . import rng
+        from .layers.flowlayer import live_capture
+        e = _TrainEntry()
+        e.device, e.params, e.frozen, e.generation, e.waiting = device, params, frozen, 0, None
+        e.x = torch.empty(x.shape, device=device, dtype=x.dtype)
+        e.ctx = None if ctx is None else torch.empty(ctx.shape, device=device, dtype=ctx.dtype)
+        with torch.no_grad():
+            e.x.copy_(x)
+            if ctx is not None:
+                e.ctx.copy_(ctx)
+        # warm-up and capture draw random numbers: the generators are put back, so that the replay of this call draws what an eager call
+        # would.  torch.autograd.grad leaves .grad alone.
+        cpu_state, cuda_state = torch.get_rng_state(), torch.cuda.get_rng_state(device)
+        cur = torch.cuda.current_stream(device)
+        side = torch.cuda.Stream(device)
+        side.wait_stream(cur)
+        with _leaf_aliases(self.model, params) as leaves:
+            with torch.cuda.stream(side):
+                for _ in range(self.warmup):
+                    out = self.model.log_prob_eager(e.x, e.ctx)
+                    torch.autograd.grad(out, leaves, torch.ones_like(out), allow_unused=True)
+                del out
+            cur.wait_stream(side)
+            torch.cuda.synchronize(device)
+            e.fwd, e.bwd = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
+            del rng._capture_host_draws[:]
+            with live_capture():
+                with torch.cuda.graph(e.fwd, stream=side):
+                    e.out = self.model.log_prob_eager(e.x, e.ctx)
+                e.host_draws = list(rng._capture_host_draws)
+                del rng._capture_host_draws[:]
+                e.dlogp = torch.empty_like(e.out)
+                # the forward's autograd graph is retained: the saved activations stay allocated between a forward and a backward replay
+                with torch.cuda.graph(e.bwd, pool=e.fwd.pool(), stream=side):
+                    grads = torch.autograd.grad(e.out, leaves, e.dlogp, retain_graph=True, allow_unused=True)
+                    e.used = [g for g in grads if g is not None]
+                    e.flat = _flatten_dense_tensors(e.used) if e.used else None
+        e.slots = [i for i, g in enumerate(grads) if g is not None]
+        e.used = [params[i] for i in e.slots]
+        torch.set_rng_state(cpu_state); torch.cuda.set_rng_state(cuda_state, device)
+        cur.wait_stream(side)
+        e.versions = self._signature(frozen)
+        return e
+
 
 class GraphedTrainStep:
     """forward + loss + backward of a training step captured in ONE CUDA graph (torch.cuda.graph around the libcfpp launches, which go to
@@ -188,7 +398,7 @@ class GraphedTrainStep:
         params = [p for p in model.parameters() if p.requires_grad]
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(side):
+        with torch.cuda.stream(side), eager_training():  # the model's own training graphs stay out of this step's warm-up
             for _ in range(warmup):                     # allocator warm-up, lazy initialisations (ActNorm flags, cached constants)
                 for p in params:
                     p.grad = None

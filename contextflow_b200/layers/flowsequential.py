@@ -23,8 +23,10 @@ class FlowSequential(nn.Module):
                 m._view_ok = True                                # as a view; the squeeze kernel reads it through the batch stride (no copy)
         import os
         self._graphed = None
-        if os.environ.get('CFPP_CUDA_GRAPHS', '0') == '1':
-            self.enable_cuda_graphs()
+        self._graphed_train = None
+        scoring, training_ = os.environ.get('CFPP_CUDA_GRAPHS', '0') == '1', os.environ.get('CFPP_CUDA_GRAPHS_TRAIN', '0') == '1'
+        if scoring or training_:
+            self.enable_cuda_graphs(scoring, training=training_)
 
     def __iter__(self):
         yield from self.sequence_modules
@@ -36,21 +38,24 @@ class FlowSequential(nn.Module):
         new = self.__class__.__new__(self.__class__)
         memo[id(self)] = new
         for k, v in self.__dict__.items():
-            if k in ('_fastpath', '_graphed', '_groups', '_replicated'):
+            if k in ('_fastpath', '_graphed', '_graphed_train', '_groups', '_replicated'):
                 continue
             new.__dict__[k] = copy.deepcopy(v, memo)
         new.__dict__['_groups'] = None
         new.__dict__['_graphed'] = None
-        if self._graphed is not None:
-            new.enable_cuda_graphs()
+        new.__dict__['_graphed_train'] = None
+        training_ = self.__dict__.get('_graphed_train') is not None
+        if self._graphed is not None or training_:
+            new.enable_cuda_graphs(self._graphed is not None, training=training_)
         return new
 
     def _apply(self, fn, *args, **kwargs):
         """.to() / .cuda() / .double(): parameters may be re-created, so captured graphs and their cached tensor list are dropped."""
         out = super()._apply(fn, *args, **kwargs)
-        g = getattr(self, '_graphed', None)
-        if g is not None:
-            g.invalidate()
+        for name in ('_graphed', '_graphed_train'):
+            g = self.__dict__.get(name)
+            if g is not None:
+                g.invalidate()
         return out
 
     def _encoder_groups(self):
@@ -108,12 +113,19 @@ class FlowSequential(nn.Module):
         # logdet = ((0 + ldj_0) + ldj_1) + ...; logprob + logdet  (flowsequential.py:20-27), same order, one launch
         return out, ops.ldj_sum(terms, B, self.mixtures, input.device, last=logprob)
 
-    def enable_cuda_graphs(self, flag: bool = True):
-        """Replay `log_prob` from a captured CUDA graph (one graph per input shape) whenever autograd is off: removes the per-launch
-        host overhead of the ~10^2 kernels of a forward.  Off by default; `python -m contextflow_b200.run` turns it on with
-        CFPP_CUDA_GRAPHS=1.  forward() (which also returns z) always runs eagerly."""
-        from ..graphed import GraphedLogProb
+    def enable_cuda_graphs(self, flag: bool = True, training: bool = False):
+        """flag: replay `log_prob` from a captured CUDA graph (one graph per input shape) whenever autograd is off: removes the
+        per-launch host overhead of the ~10^2 kernels of a forward.
+        training: also replay `log_prob` under autograd, from a forward and a backward graph per input shape (graphed.GraphedTrainLogProb),
+        for a training loop that keeps its own loss, backward() and optimizer step; the ~10^3 launches of a training step then become
+        two graph launches.  The first call at a new shape, and the first after a load_state_dict, run eagerly; the second captures.
+        Calls with an input that requires grad, with a gradient hook on a parameter, inside another capture or under a replayed noise
+        tape stay eager.
+        Both off by default; `python -m contextflow_b200.run` turns them on with CFPP_CUDA_GRAPHS=1 and CFPP_CUDA_GRAPHS_TRAIN=1.
+        forward() (which also returns z) always runs eagerly."""
+        from ..graphed import GraphedLogProb, GraphedTrainLogProb
         self._graphed = GraphedLogProb(self) if flag else None
+        self._graphed_train = GraphedTrainLogProb(self) if training else None
         return self
 
     def log_prob_eager(self, input, context=None):
@@ -157,6 +169,9 @@ class FlowSequential(nn.Module):
     def _log_prob_single(self, input, context=None):
         if torch.is_grad_enabled():
             ops.begin_training_step()
+            gt = self.__dict__.get('_graphed_train')
+            if gt is not None and input.is_cuda:
+                return gt(input, context)
         g = getattr(self, '_graphed', None)
         if g is not None and input.is_cuda and not torch.is_grad_enabled() and not torch.cuda.is_current_stream_capturing():
             from .. import rng

@@ -6,6 +6,10 @@ model.py does `from layers import *` and `from layers.rtdl.nn._embeddings import
 the reference directory, whose own `layers/` package would win on sys.path.  The replacement is therefore registered in
 sys.modules under those names BEFORE model.py executes; datasets/, utils/, config.py, experiment_*.py keep coming from
 the reference.
+
+The launcher also installs the fused AdamW (contextflow_b200/optim.py) and turns on CUDA graphs for model.log_prob: scoring calls and
+the training loop's calls (CFPP_CUDA_GRAPHS=1, CFPP_CUDA_GRAPHS_TRAIN=1 unless already set), so the unchanged loop runs a training step
+as two graph launches plus its own loss and optimizer step.
 """
 import os
 import runpy
@@ -37,8 +41,10 @@ def main(argv=None):
         raise SystemExit(__doc__)
     script = os.path.abspath(argv[0])
     # inference calls of model.log_prob (eval_epoch, experiment_ad.py:262 / experiment_cl.py:185) replay a captured CUDA graph per input
-    # shape; training calls (autograd on) always launch eagerly.  CFPP_CUDA_GRAPHS=0 in the environment keeps everything eager.
+    # shape; training calls (autograd on, train_epoch) replay a forward and a backward graph per input shape while the loop keeps its own
+    # loss, backward() and optimizer step.  CFPP_CUDA_GRAPHS=0 keeps scoring eager, CFPP_CUDA_GRAPHS_TRAIN=0 keeps training eager.
     os.environ.setdefault('CFPP_CUDA_GRAPHS', '1')
+    os.environ.setdefault('CFPP_CUDA_GRAPHS_TRAIN', '1')
     install_layers()
     if os.environ.get('CFPP_FUSED_ADAMW', '1') != '0':          # model.py:289 `optim.AdamW(...)` then builds the one-kernel optimizer
         from contextflow_b200 import optim as _optim
