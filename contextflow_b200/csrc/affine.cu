@@ -338,13 +338,11 @@ extern "C" int cfpp_conv1x1_fwd(const float* x, float* z, float* ldj, const floa
   if (B <= 0) return CFPP_OK;
   Conv1x1Args a{x, z, ldj, NN, logabsdet, c, logp_c, contextflow, an_t, an_logs, an_per_sample, an_logp_c, an_logp_scale, B, D, HW};
   a.an_stride = an_per_sample == 0 ? 0 : (an_per_sample == 1 ? D : 2 * D);
-  {   // register-tiled kernel (conv1x1_rt.cu) whenever its tile fits; CFPP_C1X1=col forces the column-per-thread kernel below
-    static int force_col = -1;
-    if (force_col < 0) { const char* v = getenv("CFPP_C1X1"); force_col = (v && v[0] == 'c') ? 1 : 0; }
+  {   // register-tiled kernel (conv1x1_rt.cu) where it measured faster and its tile fits; the column-per-thread kernel below otherwise
     // measured on B200 (B = 8192): shared matrix D=16/32/64 rt 80/57/47 us vs column kernel 61/55/59 us; per-sample matrices
     // rt 100/80/161 us vs 72/86/148 us -- the per-sample assembly of W from c dominates both; rt is used where it wins
     const bool use_rt = c ? (D > 16 && D <= 32) : (D > 32);
-    if (!force_col && use_rt) {
+    if (use_rt) {
       const int rc = cfpp_conv1x1_rt_launch(x, z, ldj, NN, logabsdet, c, logp_c, contextflow, an_t, an_logs, a.an_stride, an_logp_c, an_logp_scale,
                                             B, D, HW, (cudaStream_t)stream);
       if (rc != CFPP_ERR_UNSUPPORTED) return rc;

@@ -371,7 +371,7 @@ __global__ void __launch_bounds__(256) conv_rows_bwd_weight_kernel(const float* 
 // 128/64-bit shared loads (rows of WzP columns, a multiple of 4, so every group starts 16-byte aligned) and the 4 x 9 weights
 // W[co, ci0..ci0+3, :, :] are 36 contiguous floats = nine 128-bit warp-uniform loads; together they feed 36 TP FMAs (TP = 4: 144 FMAs per 15
 // loads, against 16 per 8 in the generic tile).  TP = 6 covers a whole padded row of a 4-wide image with one group.
-template <int TP, bool PF>
+template <int TP>
 __global__ void __launch_bounds__(256, 2) conv2d_bwd_data3_kernel(const float* __restrict__ dout, const float* __restrict__ W,
                                                                   const float* __restrict__ act, int64_t act_bstride,
                                                                   float* __restrict__ din, int64_t din_bstride, int accumulate,
@@ -425,25 +425,17 @@ __global__ void __launch_bounds__(256, 2) conv2d_bwd_data3_kernel(const float* _
     for (int c = 0; c < 4; ++c)
 #pragma unroll
       for (int j = 0; j < TP; ++j) acc[c][j] = 0.f;
-    float4 wn[9];                                              // PF: the weights of the next output channel are requested one iteration ahead
-    if (PF) {
+    float4 wn[9];                                              // the weights of the next output channel are requested one iteration ahead
 #pragma unroll
-      for (int q = 0; q < 9; ++q) wn[q] = __ldg(wq + q);
-    }
+    for (int q = 0; q < 9; ++q) wn[q] = __ldg(wq + q);
 #pragma unroll 2
     for (int co = 0; co < Cout; ++co) {                        // unrolled by two: the (w, wn) register sets swap roles instead of being copied
       float w[36];
-      if (PF) {
 #pragma unroll
-        for (int q = 0; q < 9; ++q) { w[4 * q] = wn[q].x; w[4 * q + 1] = wn[q].y; w[4 * q + 2] = wn[q].z; w[4 * q + 3] = wn[q].w; }
-        wq += co + 1 < Cout ? wstep : 0;                       // the last iteration re-reads its own row (in bounds, unused)
+      for (int q = 0; q < 9; ++q) { w[4 * q] = wn[q].x; w[4 * q + 1] = wn[q].y; w[4 * q + 2] = wn[q].z; w[4 * q + 3] = wn[q].w; }
+      wq += co + 1 < Cout ? wstep : 0;                         // the last iteration re-reads its own row (in bounds, unused)
 #pragma unroll
-        for (int q = 0; q < 9; ++q) wn[q] = __ldg(wq + q);
-      } else {
-#pragma unroll
-        for (int q = 0; q < 9; ++q) { const float4 t = __ldg(wq + q); w[4 * q] = t.x; w[4 * q + 1] = t.y; w[4 * q + 2] = t.z; w[4 * q + 3] = t.w; }
-        wq += wstep;
-      }
+      for (int q = 0; q < 9; ++q) wn[q] = __ldg(wq + q);
 #pragma unroll
       for (int kh = 0; kh < 3; ++kh) {
         const float* r = gp + (2 - kh) * WzP;
@@ -1177,14 +1169,11 @@ extern "C" int cfpp_conv2d_bwd_data(const float* dout, const float* W, const flo
     const int NG = (Wd + 2 + TP - 1) / TP, WzP = TP == 4 ? 4 * NG : 8;
     const size_t smem3 = ((size_t)Cout * (H + 4) * WzP + 4 + (size_t)Cin * odd_stride((H + 2) * (Wd + 2))) * sizeof(float);
     bool ok = false;
-    const char* ev = getenv("CFPP_BWD_DATA3");
-    const bool pf = !(ev && ev[0] == '2');                        // CFPP_BWD_DATA3=2: without the one-iteration-ahead weight loads (A/B)
-#define CFPP_BD3(TP_, PF_) do { auto kern = conv2d_bwd_data3_kernel<TP_, PF_>; \
+#define CFPP_BD3(TP_) do { auto kern = conv2d_bwd_data3_kernel<TP_>; \
       if ((ok = want_smem(kern, smem3))) { \
         cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);   /* two samples resident per SM */ \
         kern<<<B, 256, smem3, (cudaStream_t)stream>>>(dout, W, act, act_bstride, din, din_bstride, accumulate, Cin, Cout, H, Wd, NG, WzP); } } while (0)
-    if (TP == 6) { if (pf) CFPP_BD3(6, true); else CFPP_BD3(6, false); }
-    else { if (pf) CFPP_BD3(4, true); else CFPP_BD3(4, false); }
+    if (TP == 6) CFPP_BD3(6); else CFPP_BD3(4);
 #undef CFPP_BD3
     if (ok) return check_launch("conv2d_bwd_data");
   }

@@ -796,14 +796,14 @@ extern "C" int cfpp_vit_tc_fwd(const float* x, int64_t x_bstride, float* h, cons
   vt::Args a{x, x_bstride, h, d, (const uint8_t*)wpack, B, vt::kRows / d.n_tok, 0, (d.T + 15) / 16 * 16};
   a.ntiles = (B + a.S - 1) / a.S;
   const int grid = a.ntiles < num_sms() ? a.ntiles : num_sms();
-  static const bool v1 = [] { const char* e = getenv("CFPP_VIT_TC_V1"); return e && *e == '1'; }();   // the one-thread-per-row kernel, kept for A/B timing
   const size_t smem4 = vt::smem_bytes4(d.n_tok, d.depth);
-  if (!v1 && smem4 <= 227 * 1024) {
+  if (smem4 <= 227 * 1024) {
     static DeviceHighWater attr4;                               // per device: one process may drive several GPUs
     if (attr4.raise((long long)smem4)) cudaFuncSetAttribute(vt::vit_tc4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem4);
     vt::vit_tc4_kernel<<<grid, vt::kThreads4, smem4, (cudaStream_t)stream>>>(a);
     return check_launch("vit_cond_tc_fwd");
   }
+  // one thread per token row needs less shared memory: it takes the shapes whose four-threads-per-row tile does not fit
   const size_t smem = vt::smem_bytes(d.n_tok, d.depth);
   CFPP_REQUIRE(smem <= 227 * 1024, "vit_tc: depth %d does not fit the shared-memory parameter table", d.depth);
   static DeviceHighWater attr;

@@ -1,367 +1,38 @@
 // SimpleViT conditioner of TransCoupling on the tensor cores, general form: token widths T <= 192 (up to three 64-channel operand
 // panels), any number of tokens per sample up to 128 (the ATM stack: T in {36, 72, 144, 152}, 9 / 18 / 36 / 38 tokens).
 //
-// Same mapping as vit_tc.cu -- a CTA owns 128 token rows (whole samples), compute thread r is token row r, every linear layer is a set
-// of 128 x 64 x 64 tcgen05.mma groups on fp16 hi / scaled-lo operand pairs (fp32 faithful), weights stream through a bulk-TMA ring --
-// with the three things that stop fitting in registers / one panel handled as follows:
-//   * the residual stream x (T <= 192 floats per row) lives in shared memory (row stride = 4 mod 8 floats: conflict-free 128-bit
-//     row access by consecutive lanes); the thread walks its row in 64-wide register chunks;
-//   * a GEMM with K = T has P = ceil(T / 64) operand panels and N = T output chunks: the MMA issuer walks (output chunk, K panel),
-//     accumulating the panels of a chunk into one 128-column TMEM block (main | scaled cross products); one 16 KB weight chunk per
-//     (output chunk, K panel);
-//   * keys / values of a sample may belong to rows of other warps: they are staged in the operand panels 1-2 (free between the q,k,v
-//     GEMMs and the next LayerNorm) and published with a named barrier of the compute threads.
-// LayerNorm / bias rows of the current layer are staged in shared memory once per layer.
+// A CTA owns 128 token rows (whole samples); every linear layer is a set of 128 x 64 x 64 tcgen05.mma groups on fp16 hi / scaled-lo
+// operand pairs (fp32 faithful), weights stream through a bulk-TMA ring.  A GEMM with K = T has P = ceil(T / 64) operand panels and
+// N = T output chunks: the MMA issuer walks (output chunk, K panel), accumulating the panels of a chunk into one 128-column TMEM block
+// (main | scaled cross products); one 16 KB weight chunk per (output chunk, K panel).
+//
+// Four threads per token row (the layout of vit_tc4 in vit_tc.cu): 16 compute warps share the tile, warp w serves TMEM lane quadrant
+// w % 4 and column group g = w / 4, i.e. columns 16 g .. +15 of EVERY 64-wide chunk.  (With one thread per row a scheduler has one compute
+// warp and nothing to switch to while a TMEM load or the MMA round trip is outstanding.)  The residual stream is P x 16 registers per
+// thread (no row buffer in shared memory: the ring gets the space); row-wide sums cross the four column groups through shared memory under
+// a per-quadrant named barrier.  The attention runs on the tensor cores as well: S = q k^T over the whole tile (128 x 128, only a sample's
+// own block is used), softmax in registers (32 key columns per thread), O = P v with v^T staged as a B operand; q / k / v and the
+// probabilities use the operand panels, which are free between the q,k,v GEMM and the next LayerNorm.  LayerNorm / bias rows of the
+// current layer are staged in shared memory once per layer.
 #include "vit_tc_helpers.cuh"
-#include <cstdlib>
 
 namespace cfpp {
 namespace vt2 {
 using namespace vtx;
 
 constexpr int kRows = 128, kPanels = 3;
-constexpr int kThreads = 192, kMaxStages = 8;       // ring slots: as many 16 KB weight chunks as the shared memory left by the tile allows
+constexpr int kMaxStages = 8;                       // ring slots: as many 16 KB weight chunks as the shared memory left by the tile allows
 constexpr int kChunkBytes = 2 * kW * 128;           // [hi image 64 rows x 128 B][lo image]
 constexpr int kPanelBytes = 2 * kRows * 128;        // hi rows + lo rows of one 64-channel operand panel
 
 struct Args {
-  const float* x; int64_t x_bstride; float* h; cfpp_vit_desc d; const uint8_t* wpack; int B, S, ntiles, NPT, P, PD, XS, nstages, xrows;
+  const float* x; int64_t x_bstride; float* h; cfpp_vit_desc d; const uint8_t* wpack; int B, S, ntiles, NPT, P, PD, nstages;
 };
 
 enum { BAR_FULL = 0, BAR_EMPTY = kMaxStages, BAR_AREADY = 2 * kMaxStages, BAR_ACC, BAR_COUNT };
 
-__device__ __forceinline__ void compute_sync() { asm volatile("bar.sync 1, 128;" ::: "memory"); }   // the 128 compute threads
-
-// 64-wide chunk c of the thread's x row (zero beyond T; T % 4 == 0)
-__device__ __forceinline__ void load_x_chunk(const float* xrow, int c, int T, float (&v)[kW]) {
-#pragma unroll
-  for (int q = 0; q < 16; ++q) {
-    const int col = 64 * c + 4 * q;
-    float4 t = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (col < T) t = *reinterpret_cast<const float4*>(xrow + col);
-    v[4 * q] = t.x; v[4 * q + 1] = t.y; v[4 * q + 2] = t.z; v[4 * q + 3] = t.w;
-  }
-}
-__device__ __forceinline__ void store_x_chunk(float* xrow, int c, int T, const float (&v)[kW]) {
-#pragma unroll
-  for (int q = 0; q < 16; ++q) {
-    const int col = 64 * c + 4 * q;
-    if (col < T) *reinterpret_cast<float4*>(xrow + col) = make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
-  }
-}
-// LayerNorm statistics (eps 1e-5) of the first n entries of the row (two passes over shared memory)
-__device__ __forceinline__ void ln_stats(const float* xrow, int n, float& mean, float& rstd) {
-  if (n & 3) {                                               // odd widths (patch_dim = 18): scalar passes
-    float s = 0.f;
-    for (int i = 0; i < n; ++i) s += xrow[i];
-    mean = s / (float)n;
-    float v = 0.f;
-    for (int i = 0; i < n; ++i) { const float dd = xrow[i] - mean; v = fmaf(dd, dd, v); }
-    rstd = 1.0f / sqrtf(v / (float)n + 1e-5f);
-    return;
-  }
-  float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
-  for (int i = 0; i < n; i += 4) { const float4 t = *reinterpret_cast<const float4*>(xrow + i); s0 += t.x; s1 += t.y; s2 += t.z; s3 += t.w; }
-  mean = ((s0 + s1) + (s2 + s3)) / (float)n;
-  float v0 = 0.f, v1 = 0.f, v2 = 0.f, v3 = 0.f;
-  for (int i = 0; i < n; i += 4) {
-    const float4 t = *reinterpret_cast<const float4*>(xrow + i);
-    const float d0 = t.x - mean, d1 = t.y - mean, d2 = t.z - mean, d3 = t.w - mean;
-    v0 = fmaf(d0, d0, v0); v1 = fmaf(d1, d1, v1); v2 = fmaf(d2, d2, v2); v3 = fmaf(d3, d3, v3);
-  }
-  rstd = 1.0f / sqrtf(((v0 + v1) + (v2 + v3)) / (float)n + 1e-5f);
-}
-
-__global__ void __launch_bounds__(kThreads, 1) vit_tc2_kernel(const Args a) {
-  extern __shared__ __align__(1024) uint8_t vt2_smem_raw[];
-  uint8_t* base = vt2_smem_raw + ((1024u - (smem_u32(vt2_smem_raw) & 1023u)) & 1023u);   // (pointer arithmetic on the shared array keeps the address space)
-  uint8_t* ops = base;                                        // kPanels x [hi 128 rows x 128 B][lo]
-  uint8_t* ring = ops + kPanels * kPanelBytes;                // nstages x kChunkBytes
-  const int kStages = a.nstages;
-  float* X = reinterpret_cast<float*>(ring + kStages * kChunkBytes);       // [xrows][XS]: only the rows that hold tokens
-  float* lprm = X + a.xrows * a.XS;                             // [6][P * 64]: lna_w lna_b lnf_w lnf_b b1 b2 of the current layer, zero padded
-  const int PW = a.P * kW;
-  const uint32_t bars = smem_u32(lprm + 6 * PW);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(lprm + 6 * PW) + 2 * BAR_COUNT;
-  float* Ks = reinterpret_cast<float*>(ops + 1 * kPanelBytes);             // [128][64] fp32, aliases operand panel 1
-  float* Vs = reinterpret_cast<float*>(ops + 2 * kPanelBytes);             // aliases operand panel 2
-  auto bar = [&](int i) { return bars + 8u * i; };
-  const cfpp_vit_desc& d = a.d;
-  const int tid = threadIdx.x, warp = tid >> 5;
-  const int T = d.T, ntok = d.n_tok, depth = d.depth, P = a.P, PD = a.PD, XS = a.XS;
-
-  if (tid == 0) {
-    for (int i = 0; i < kStages; ++i) { mbar_init(bar(BAR_FULL + i), 1); mbar_init(bar(BAR_EMPTY + i), 1); }
-    mbar_init(bar(BAR_AREADY), kRows); mbar_init(bar(BAR_ACC), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 4) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-
-  // weight chunks per tile, in consumption order: embed (P x PD), per layer qkv (3 x P), out (P x 1), mlp1 (P x P), mlp2 (P x P)
-  const int chunks_per_tile = P * PD + depth * (3 * P + P + 2 * P * P);
-  const int my_tiles = (a.ntiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
-
-  if (warp == 5) {
-    if (elect_one()) {
-      uint32_t st = 0, ph = 0;
-      for (int it = 0; it < my_tiles; ++it)
-        for (int c = 0; c < chunks_per_tile; ++c) {
-          mbar_wait(bar(BAR_EMPTY + st), ph ^ 1);
-          mbar_expect_tx(bar(BAR_FULL + st), kChunkBytes);
-          bulk_g2s(smem_u32(ring + (size_t)st * kChunkBytes), a.wpack + (size_t)c * kChunkBytes, kChunkBytes, bar(BAR_FULL + st));
-          if (++st == kStages) { st = 0; ph ^= 1; }
-        }
-    }
-  } else if (warp == 4) {
-    if (elect_one()) {
-      const uint32_t id128 = make_idesc(2 * kW), id64 = make_idesc(kW);
-      const uint64_t a0 = make_desc(smem_u32(ops)), b0 = make_desc(smem_u32(ring));
-      uint32_t st = 0, ph = 0, na = 0;
-      // one GEMM: NC output chunks x PK operand panels
-      auto gemm = [&](int NC, int PK) {
-        mbar_wait(bar(BAR_AREADY), na & 1); ++na;
-        tc_fence_after();
-        for (int n = 0; n < NC; ++n)
-          for (int p = 0; p < PK; ++p) {
-            mbar_wait(bar(BAR_FULL + st), ph);
-            tc_fence_after();
-            const uint64_t bd = b0 + (uint64_t)(st * (kChunkBytes >> 4));
-            const uint64_t ah = a0 + (uint64_t)(p * (kPanelBytes >> 4)), al = ah + (uint64_t)((kRows * 128) >> 4);
-            const uint32_t dd = tmem + n * 2 * kW;
-#pragma unroll
-            for (int ks = 0; ks < 4; ++ks) {
-              mma_f16(dd, ah + 2 * ks, bd + 2 * ks, id128, (p | ks) ? 1u : 0u);
-              mma_f16(dd + kW, al + 2 * ks, bd + 2 * ks, id64, 1u);
-            }
-            tc_commit(bar(BAR_EMPTY + st));
-            if (++st == kStages) { st = 0; ph ^= 1; }
-          }
-        tc_commit(bar(BAR_ACC));
-      };
-      for (int it = 0; it < my_tiles; ++it) {
-        gemm(P, PD);
-        for (int l = 0; l < depth; ++l) { gemm(3, P); gemm(P, 1); gemm(P, P); gemm(P, P); }
-      }
-    }
-  } else {
-    const int r = tid;
-    const int HW = d.H * d.W, tw = d.W / d.p2, Cout = T / (d.p1 * d.p2);
-    const int64_t lstride = 4 * (int64_t)T + (int64_t)T * 192 + 64 * (int64_t)a.NPT + 2 * (int64_t)T * a.NPT + 2 * (int64_t)a.NPT;
-    const uint32_t trow = tmem + ((uint32_t)((warp & 3) * 32) << 16);
-    const bool rowok = r < a.xrows;                                 // rows beyond the tile's tokens own no x row: they read row 0 and never write
-    float* xrow = X + (rowok ? r : 0) * XS;
-    uint32_t nacc = 0;
-    auto a_ready = [&]() { fence_async_smem(); mbar_arrive(bar(BAR_AREADY)); };
-    auto acc_wait = [&]() { mbar_wait(bar(BAR_ACC), nacc & 1); ++nacc; tc_fence_after(); };
-    auto op_hi = [&](int p) { return ops + p * kPanelBytes; };
-    auto op_lo = [&](int p) { return ops + p * kPanelBytes + kRows * 128; };
-    // LayerNorm of the row (first n entries) with weight / bias rows w, b (zero beyond n), written as operand panels 0 .. np-1
-    auto ln_to_operands = [&](int n, int np, const float* w, const float* b, bool w_global) {
-      float mean, rstd;
-      ln_stats(xrow, n, mean, rstd);
-      for (int c = 0; c < np; ++c) {
-        float v[kW];
-        load_x_chunk(xrow, c, n, v);
-#pragma unroll
-        for (int i = 0; i < kW; ++i) {
-          const int col = 64 * c + i;
-          const float wv = w_global ? (col < n ? __ldg(w + col) : 0.f) : w[col], bv = w_global ? (col < n ? __ldg(b + col) : 0.f) : b[col];
-          v[i] = col < n ? fmaf((v[i] - mean) * rstd, wv, bv) : 0.f;
-        }
-        store_operand_row(op_hi(c), op_lo(c), r, v);
-      }
-    };
-    for (int it = 0; it < my_tiles; ++it) {
-      const int tile = blockIdx.x + it * gridDim.x;
-      const int b0 = tile * a.S;
-      const int s = r / ntok, tok = r - s * ntok;
-      const bool live = r < a.S * ntok && b0 + s < a.B;
-      const int th = tok / tw, tww = tok - th * tw;
-      // ---- patchify into the row buffer, LayerNorm(patch_dim) -> operands, Linear, + bias, LayerNorm(T), + positional embedding ----
-      for (int f = 0; f < d.patch_dim; ++f) {
-        float v = 0.f;
-        if (live) {
-          const int c = f % d.Cin, pp = f / d.Cin, i = pp / d.p2, j = pp - i * d.p2;
-          v = __ldg(a.x + (int64_t)(b0 + s) * a.x_bstride + (int64_t)c * HW + (th * d.p1 + i) * d.W + (tww * d.p2 + j));
-        }
-        if (rowok) xrow[f] = v;
-      }
-      ln_to_operands(d.patch_dim, PD, d.ln0_w, d.ln0_b, true);
-      a_ready();
-      acc_wait();
-      for (int c = 0; c < P; ++c) {
-        float v[kW];
-        load_acc_row(trow + c * 2 * kW, v);
-#pragma unroll
-        for (int i = 0; i < kW; ++i) { const int col = 64 * c + i; v[i] += col < T ? __ldg(d.pe_b + col) : 0.f; }
-        if (rowok) store_x_chunk(xrow, c, T, v);
-      }
-      tc_fence_before();
-      {
-        float mean, rstd;
-        ln_stats(xrow, T, mean, rstd);
-        if (rowok) for (int i = 0; i < T; ++i) xrow[i] = fmaf((xrow[i] - mean) * rstd, __ldg(d.ln1_w + i), __ldg(d.ln1_b + i)) + __ldg(d.pos + tok * T + i);
-      }
-
-      for (int l = 0; l < depth; ++l) {
-        // ---- this layer's LayerNorm / bias rows -> shared memory ----
-        compute_sync();                                              // everyone is done with the previous layer's rows
-        {
-          const float* Lp = d.layers + l * lstride;
-          const float* lnf = Lp + 2 * T + (int64_t)T * 192 + 64 * (int64_t)a.NPT;
-          const float* b1 = lnf + 2 * T + (int64_t)T * a.NPT;
-          const float* b2 = b1 + a.NPT + (int64_t)T * a.NPT;
-          for (int idx = r; idx < 6 * PW; idx += kRows) {
-            const int k = idx / PW, i = idx - k * PW;
-            const float* src = k == 0 ? Lp : k == 1 ? Lp + T : k == 2 ? lnf : k == 3 ? lnf + T : k == 4 ? b1 : b2;
-            lprm[idx] = i < T ? __ldg(src + i) : 0.f;
-          }
-        }
-        compute_sync();
-        // ---- attention: x += Wo softmax(q k^T / 8) v ----
-        ln_to_operands(T, P, lprm, lprm + PW, false);
-        a_ready();
-        acc_wait();
-        float q[kW];
-        {
-          float kv[kW];
-          load_acc_row(trow + 2 * kW, kv);                            // k -> staging (operand panel 1 is free now)
-          // rows are 256 bytes apart: 16-byte piece q of row r is stored at position q ^ (r % 16), so that the lanes of a warp (consecutive
-          // rows, same q) hit different banks; readers apply the same XOR
-#pragma unroll
-          for (int i = 0; i < 16; ++i) *reinterpret_cast<float4*>(Ks + r * kW + 4 * (i ^ (r & 15))) = make_float4(kv[4 * i], kv[4 * i + 1], kv[4 * i + 2], kv[4 * i + 3]);
-          load_acc_row(trow + 4 * kW, kv);                            // v
-#pragma unroll
-          for (int i = 0; i < 16; ++i) *reinterpret_cast<float4*>(Vs + r * kW + 4 * (i ^ (r & 15))) = make_float4(kv[4 * i], kv[4 * i + 1], kv[4 * i + 2], kv[4 * i + 3]);
-        }
-        load_acc_row(trow, q);
-        tc_fence_before();
-        compute_sync();                                               // keys / values of the sample may be rows of other warps
-        {
-          float o[kW];
-#pragma unroll
-          for (int i = 0; i < kW; ++i) o[i] = 0.f;
-          if (live) {
-            float mx = -INFINITY, den = 0.f;
-            const int r0 = r - tok;
-            for (int j = 0; j < ntok; ++j) {
-              const int rj = r0 + j, sw = rj & 15;
-              const float* kr = Ks + rj * kW;
-              float d0 = 0.f, d1 = 0.f, d2 = 0.f, d3 = 0.f;
-#pragma unroll
-              for (int qq = 0; qq < 16; ++qq) {
-                const float4 k4 = *reinterpret_cast<const float4*>(kr + 4 * (qq ^ sw));
-                d0 = fmaf(q[4 * qq], k4.x, d0); d1 = fmaf(q[4 * qq + 1], k4.y, d1); d2 = fmaf(q[4 * qq + 2], k4.z, d2); d3 = fmaf(q[4 * qq + 3], k4.w, d3);
-              }
-              const float dot = ((d0 + d1) + (d2 + d3)) * 0.125f;
-              if (dot > mx) {                                           // a new running maximum (rare after the first keys): rescale what was accumulated
-                const float corr = __expf(mx - dot);
-                den *= corr;
-#pragma unroll
-                for (int i = 0; i < kW; ++i) o[i] *= corr;
-                mx = dot;
-              }
-              const float pj = __expf(dot - mx);
-              den += pj;
-              const float* vr = Vs + rj * kW;
-#pragma unroll
-              for (int qq = 0; qq < 16; ++qq) {
-                const float4 v4 = *reinterpret_cast<const float4*>(vr + 4 * (qq ^ sw));
-                o[4 * qq] = fmaf(pj, v4.x, o[4 * qq]); o[4 * qq + 1] = fmaf(pj, v4.y, o[4 * qq + 1]);
-                o[4 * qq + 2] = fmaf(pj, v4.z, o[4 * qq + 2]); o[4 * qq + 3] = fmaf(pj, v4.w, o[4 * qq + 3]);
-              }
-            }
-            const float inv = 1.0f / den;
-#pragma unroll
-            for (int i = 0; i < kW; ++i) o[i] *= inv;
-          }
-          store_operand_row(op_hi(0), op_lo(0), r, o);               // panel 0 does not overlap the k / v staging (panels 1-2)
-        }
-        a_ready();
-        acc_wait();                                                    // (all compute threads have arrived: nobody still reads k / v)
-        for (int c = 0; c < P; ++c) {
-          float v[kW], xv[kW];
-          load_acc_row(trow + c * 2 * kW, v);
-          load_x_chunk(xrow, c, T, xv);
-#pragma unroll
-          for (int i = 0; i < kW; ++i) xv[i] += v[i];
-          if (rowok) store_x_chunk(xrow, c, T, xv);
-        }
-        tc_fence_before();
-        // ---- MLP: x += W2 gelu(W1 LN(x) + b1) + b2 ----
-        ln_to_operands(T, P, lprm + 2 * PW, lprm + 3 * PW, false);
-        a_ready();
-        acc_wait();
-        for (int c = 0; c < P; ++c) {
-          float v[kW];
-          load_acc_row(trow + c * 2 * kW, v);
-          const float* pb1 = lprm + 4 * PW + 64 * c;
-#pragma unroll
-          for (int i = 0; i < kW; ++i) { const float u = v[i] + pb1[i]; v[i] = 0.5f * u * (1.0f + erf_as(u * 0.70710678118654752440f)); }
-          store_operand_row(op_hi(c), op_lo(c), r, v);                // hidden chunk c = operand panel c of the second MLP layer
-        }
-        tc_fence_before();
-        a_ready();
-        acc_wait();
-        for (int c = 0; c < P; ++c) {
-          float v[kW], xv[kW];
-          load_acc_row(trow + c * 2 * kW, v);
-          load_x_chunk(xrow, c, T, xv);
-          const float* pb2 = lprm + 5 * PW + 64 * c;
-#pragma unroll
-          for (int i = 0; i < kW; ++i) xv[i] += v[i] + pb2[i];
-          if (rowok) store_x_chunk(xrow, c, T, xv);
-        }
-        tc_fence_before();
-      }
-      // ---- final LayerNorm, un-patchify 'b (h w) (p1 p2 c) -> b c (h p1) (w p2)' ----
-      {
-        float mean, rstd;
-        ln_stats(xrow, T, mean, rstd);
-        if (live)
-          for (int f = 0; f < T; ++f) {
-            const int c = f % Cout, pp = f / Cout, i = pp / d.p2, j = pp - i * d.p2;
-            a.h[((int64_t)(b0 + s) * Cout + c) * HW + (th * d.p1 + i) * d.W + (tww * d.p2 + j)] =
-                fmaf((xrow[f] - mean) * rstd, __ldg(d.lnf_w + f), __ldg(d.lnf_b + f));
-          }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 4) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512) : "memory");
-}
-
-static int xs_of(int T) { int xs = (T + 3) & ~3; while ((xs & 7) != 4) xs += 4; return xs; }
-static size_t fixed_bytes(int T, int P, int xrows) {
-  return 1024 + (size_t)kPanels * kPanelBytes + (size_t)xrows * xs_of(T) * 4 + (size_t)6 * P * kW * 4 + BAR_COUNT * 8 + 64;
-}
-static int stages_for(int T, int P, int xrows) {
-  const long long left = 227LL * 1024 - (long long)fixed_bytes(T, P, xrows);
-  long long n = left / kChunkBytes;
-  return (int)(n > kMaxStages ? kMaxStages : n);
-}
-
-
-// ---------------------------------------------------------------------------------------------------------------------------------------
-// Four threads per token row (the layout of vit_tc4 in vit_tc.cu, for T <= 192 and up to 64 tokens per sample).  The kernel above keeps a
-// whole row in ONE thread -- 4 compute warps per SM, one per scheduler, nothing to switch to while a TMEM load or the MMA round trip is
-// outstanding (cfg3: 0.02-0.03 of the tensor peak, 85 % of the step).  Here 16 compute warps share the tile: warp w serves TMEM lane quadrant
-// w % 4 and column group g = w / 4, i.e. columns 16 g .. +15 of EVERY 64-wide chunk; the residual stream shrinks to P x 16 registers per
-// thread (no row buffer in shared memory), row-wide sums cross the four column groups through shared memory under a per-quadrant named
-// barrier, q rows are staged in shared memory, k / v rows in operand panels 1-2 (free between the q,k,v GEMM and the next LayerNorm), the
-// attention scores in operand panel 0 (free until the attention output is written there; one CTA-wide barrier separates the two uses).
-// Weight stream, MMA issue order and the fp16 hi / scaled-lo arithmetic are those of the kernel above: the two are interchangeable.
 constexpr int kCG = 4, kCW = kW / kCG;
 constexpr int kThreads5 = (4 * kCG + 2) * 32;
-constexpr int kQStride = 68;
 
 __device__ __forceinline__ uint64_t pack2(float a, float b) { uint64_t r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(a), "f"(b)); return r; }
 __device__ __forceinline__ void unpack2(uint64_t v, float& a, float& b) { asm("mov.b64 {%0, %1}, %2;" : "=f"(a), "=f"(b) : "l"(v)); }
@@ -476,10 +147,7 @@ __device__ __forceinline__ void store_p32(uint8_t* ops, int row, int g, const fl
 
 enum { G_LN0W = 0, G_LN0B, G_PEB, G_LN1W, G_LN1B, G_LNFW, G_LNFB, G_ROWS };
 
-// TCA: attention on the tensor cores as well -- S = q k^T over the whole tile (128 x 128, only a sample's own block is used), softmax in
-// registers (32 key columns per thread), O = P v with v^T staged as a B operand; the FP32 form (TCA = false) stages q / k / v / scores in
-// shared memory and is bound by shared-memory bandwidth at 36-38 tokens per sample
-template <int P, bool TCA>
+template <int P>
 __global__ void __launch_bounds__(kThreads5, 1) vit_tc5_kernel(const Args a) {
   extern __shared__ __align__(1024) uint8_t vt5_smem_raw[];
   uint8_t* base = vt5_smem_raw + ((1024u - (smem_u32(vt5_smem_raw) & 1023u)) & 1023u);   // pointer arithmetic on the shared array keeps the address space (LDS / STS, not generic LD / ST)
@@ -487,17 +155,13 @@ __global__ void __launch_bounds__(kThreads5, 1) vit_tc5_kernel(const Args a) {
   uint8_t* ops = base;                                        // kPanels x [hi 128 rows x 128 B][lo]
   uint8_t* ring = ops + kPanels * kPanelBytes;                // nstages x kChunkBytes
   const int kStages = a.nstages;
-  float* Qs = reinterpret_cast<float*>(ring + kStages * kChunkBytes);      // [128][kQStride] (FP32 attention only)
-  float* red2 = Qs + (TCA ? 0 : kRows * kQStride);            // [2][kCG][128] row-reduction partials
+  float* red2 = reinterpret_cast<float*>(ring + kStages * kChunkBytes);    // [2][kCG][128] row-reduction partials
   float* lprm = red2 + 2 * kCG * kRows;                       // [6][PW]: lna_w lna_b lnf_w lnf_b b1 b2 of the current layer, zero padded
   float* gprm = lprm + 6 * PW;                                // [G_ROWS][PW]: ln0 w/b (patch_dim wide), pe_b, ln1 w/b, final norm w/b
   int* foff_in = reinterpret_cast<int*>(gprm + G_ROWS * PW);  // [PW] feature part of the patchify offset; -1 beyond patch_dim
   int* foff_out = foff_in + PW;                               // [PW] the same for the output h; -1 beyond T
   const uint32_t bars = smem_u32(foff_out + PW);
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(foff_out + PW) + 2 * BAR_COUNT;
-  float* Sc = reinterpret_cast<float*>(ops);                  // [128][64] attention scores, aliases operand panel 0; column j of row r sits at j ^ (r & 31)
-  float* Ks = reinterpret_cast<float*>(ops + 1 * kPanelBytes);             // [128][64] fp32, aliases operand panel 1
-  float* Vs = reinterpret_cast<float*>(ops + 2 * kPanelBytes);             // aliases operand panel 2
   auto bar = [&](int i) { return bars + 8u * i; };
   const cfpp_vit_desc& d = a.d;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -577,7 +241,7 @@ __global__ void __launch_bounds__(kThreads5, 1) vit_tc5_kernel(const Args a) {
         gemm(P, PD);
         for (int l = 0; l < depth; ++l) {
           gemm(3, P);
-          if (TCA) {
+          {
             const uint64_t ah = a0, al = a0 + (uint64_t)((kRows * 128) >> 4), bk = a0 + (uint64_t)(kPanelBytes >> 4);
             // S = q k^T: A = q rows (panel 0), B = k rows (panel 1: 128 hi rows | 128 lo rows); main block columns 0-127, cross block 128-255
             mbar_wait(bar(BAR_AREADY), na & 1); ++na;
@@ -717,124 +381,48 @@ __global__ void __launch_bounds__(kThreads5, 1) vit_tc5_kernel(const Args a) {
         a_ready();
         acc_wait();
         float o[kCW];
-        if (TCA) {
-          const int r0 = r - tok;
-          {
-            float t16[kCW];
-            load_acc16(trow + 2 * kW, g, t16);                      // k -> B-operand rows (panel 1)
-            store_operand16(op_hi(1), op_lo(1), r, g, t16);
-            load_acc16(trow + 4 * kW, g, t16);                      // v -> v^T (panel 2)
-            store_vt16(ops + 2 * kPanelBytes, r, g, t16);
-            load_acc16(trow, g, t16);                               // q -> A-operand rows (panel 0)
-            store_operand16(op_hi(0), op_lo(0), r, g, t16);
-          }
-          tc_fence_before();
-          a_ready();
-          acc_wait();                                               // S = q k^T
-          float pv[32];
-#pragma unroll
-          for (int h = 0; h < 2; ++h) {
-            float v[16], u[16];
-            tmem_ld16(trow + 32 * g + 16 * h, v);
-            tmem_ld16(trow + 2 * kW + 32 * g + 16 * h, u);
-            tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 16; ++i) pv[16 * h + i] = fmaf(u[i], kLoInv, v[i]) * 0.125f;   // dim_head ** -0.5
-          }
-          tc_fence_before();
-          const int jlo = r0 - 32 * g, jhi = jlo + ntok;            // this thread's key columns i with jlo <= i < jhi belong to the row's sample
-          float mx = -INFINITY;
-#pragma unroll
-          for (int i = 0; i < 32; ++i) { if (!(live && i >= jlo && i < jhi)) pv[i] = -INFINITY; mx = fmaxf(mx, pv[i]); }
-          mx = row_max5(mx, red2 + (flip & 1) * kCG * kRows, r, g, quad); ++flip;
-          if (!live) mx = 0.f;
-          float den = 0.f;
-#pragma unroll
-          for (int i = 0; i < 32; ++i) { pv[i] = __expf(pv[i] - mx); den += pv[i]; }
-          den = row_sum5(den, red2 + (flip & 1) * kCG * kRows, r, g, quad); ++flip;
-          const float inv = live ? 1.0f / den : 0.f;
-#pragma unroll
-          for (int i = 0; i < 32; ++i) pv[i] *= inv;
-          store_p32(ops, r, g, pv);
-          a_ready();
-          acc_wait();                                               // O = P v
-          load_acc16(trow + 6 * kW, g, o);
-          tc_fence_before();
-        } else {
+        const int r0 = r - tok;
         {
-            float t16[kCW];
-            load_acc16(trow + 2 * kW, g, t16);                        // k: 16-byte piece q of row r is stored at position q ^ (r % 16) (see the kernel above)
-#pragma unroll
-            for (int q = 0; q < 4; ++q) *reinterpret_cast<float4*>(Ks + r * kW + 4 * ((4 * g + q) ^ (r & 15))) = make_float4(t16[4 * q], t16[4 * q + 1], t16[4 * q + 2], t16[4 * q + 3]);
-            load_acc16(trow + 4 * kW, g, t16);                        // v
-#pragma unroll
-            for (int q = 0; q < 4; ++q) *reinterpret_cast<float4*>(Vs + r * kW + 4 * ((4 * g + q) ^ (r & 15))) = make_float4(t16[4 * q], t16[4 * q + 1], t16[4 * q + 2], t16[4 * q + 3]);
-            load_acc16(trow, g, t16);                                 // q
-#pragma unroll
-            for (int q = 0; q < 4; ++q) *reinterpret_cast<float4*>(Qs + r * kQStride + c0 + 4 * q) = make_float4(t16[4 * q], t16[4 * q + 1], t16[4 * q + 2], t16[4 * q + 3]);
-          }
-          tc_fence_before();
-          compute_sync5();                                            // keys / values of the sample may be rows of other quadrants
-          const int r0 = r - tok;
-          if (live) {
-            // full-width scores of the keys this column group owns (j = g, g + 4, ...), five keys per pass: a 16-byte piece of the q row is
-            // loaded once per pass instead of once per key (19 instead of 32 shared loads per key: the loop is bound by shared-memory bandwidth)
-            constexpr int NK = 5;
-            const float* qr = Qs + r * kQStride;
-            for (int jb = g; jb < ntok; jb += kCG * NK) {
-              float acc[NK][4];
-              const float* kr[NK]; int sw[NK];
-#pragma unroll
-              for (int u = 0; u < NK; ++u) {
-                const int j = min(jb + kCG * u, ntok - 1);             // (keys beyond the last one recompute it; not stored)
-                const int rj = r0 + j;
-                kr[u] = Ks + rj * kW; sw[u] = rj & 15;
-                acc[u][0] = acc[u][1] = acc[u][2] = acc[u][3] = 0.f;
-              }
-#pragma unroll
-              for (int q = 0; q < 16; ++q) {
-                const float4 q4 = *reinterpret_cast<const float4*>(qr + 4 * q);
-#pragma unroll
-                for (int u = 0; u < NK; ++u) {
-                  const float4 k4 = *reinterpret_cast<const float4*>(kr[u] + 4 * (q ^ sw[u]));
-                  acc[u][0] = fmaf(q4.x, k4.x, acc[u][0]); acc[u][1] = fmaf(q4.y, k4.y, acc[u][1]);
-                  acc[u][2] = fmaf(q4.z, k4.z, acc[u][2]); acc[u][3] = fmaf(q4.w, k4.w, acc[u][3]);
-                }
-              }
-#pragma unroll
-              for (int u = 0; u < NK; ++u) {
-                const int j = jb + kCG * u;
-                if (j < ntok) Sc[r * kW + (j ^ (r & 31))] = ((acc[u][0] + acc[u][1]) + (acc[u][2] + acc[u][3])) * 0.125f;   // dim_head ** -0.5
-              }
-            }
-          }
-          quad_sync5(quad);                                           // the scores of a row are written and read by its own four threads
-#pragma unroll
-          for (int i = 0; i < kCW; ++i) o[i] = 0.f;
-          if (live) {
-            const float* sr = Sc + r * kW;
-            const int sx = r & 31;
-            float mx = -INFINITY;
-            for (int j = 0; j < ntok; ++j) mx = fmaxf(mx, sr[j ^ sx]);
-            float den = 0.f;
-            for (int j = 0; j < ntok; ++j) {
-              const float pj = __expf(sr[j ^ sx] - mx);
-              den += pj;
-              const int rj = r0 + j, sw = rj & 15;
-              const float* vr = Vs + rj * kW;
-#pragma unroll
-              for (int q = 0; q < 4; ++q) {
-                const float4 v4 = *reinterpret_cast<const float4*>(vr + 4 * ((4 * g + q) ^ sw));
-                o[4 * q] = fmaf(pj, v4.x, o[4 * q]); o[4 * q + 1] = fmaf(pj, v4.y, o[4 * q + 1]);
-                o[4 * q + 2] = fmaf(pj, v4.z, o[4 * q + 2]); o[4 * q + 3] = fmaf(pj, v4.w, o[4 * q + 3]);
-              }
-            }
-            const float inv = 1.0f / den;
-#pragma unroll
-            for (int i = 0; i < kCW; ++i) o[i] *= inv;
-          }
-          compute_sync5();                                            // every score has been read: panel 0 takes the attention output
+          float t16[kCW];
+          load_acc16(trow + 2 * kW, g, t16);                      // k -> B-operand rows (panel 1)
+          store_operand16(op_hi(1), op_lo(1), r, g, t16);
+          load_acc16(trow + 4 * kW, g, t16);                      // v -> v^T (panel 2)
+          store_vt16(ops + 2 * kPanelBytes, r, g, t16);
+          load_acc16(trow, g, t16);                               // q -> A-operand rows (panel 0)
+          store_operand16(op_hi(0), op_lo(0), r, g, t16);
         }
+        tc_fence_before();
+        a_ready();
+        acc_wait();                                               // S = q k^T
+        float pv[32];
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          float v[16], u[16];
+          tmem_ld16(trow + 32 * g + 16 * h, v);
+          tmem_ld16(trow + 2 * kW + 32 * g + 16 * h, u);
+          tmem_ld_wait();
+#pragma unroll
+          for (int i = 0; i < 16; ++i) pv[16 * h + i] = fmaf(u[i], kLoInv, v[i]) * 0.125f;   // dim_head ** -0.5
+        }
+        tc_fence_before();
+        const int jlo = r0 - 32 * g, jhi = jlo + ntok;            // this thread's key columns i with jlo <= i < jhi belong to the row's sample
+        float mx = -INFINITY;
+#pragma unroll
+        for (int i = 0; i < 32; ++i) { if (!(live && i >= jlo && i < jhi)) pv[i] = -INFINITY; mx = fmaxf(mx, pv[i]); }
+        mx = row_max5(mx, red2 + (flip & 1) * kCG * kRows, r, g, quad); ++flip;
+        if (!live) mx = 0.f;
+        float den = 0.f;
+#pragma unroll
+        for (int i = 0; i < 32; ++i) { pv[i] = __expf(pv[i] - mx); den += pv[i]; }
+        den = row_sum5(den, red2 + (flip & 1) * kCG * kRows, r, g, quad); ++flip;
+        const float inv = live ? 1.0f / den : 0.f;
+#pragma unroll
+        for (int i = 0; i < 32; ++i) pv[i] *= inv;
+        store_p32(ops, r, g, pv);
+        a_ready();
+        acc_wait();                                               // O = P v
+        load_acc16(trow + 6 * kW, g, o);
+        tc_fence_before();
         store_operand16(op_hi(0), op_lo(0), r, g, o);
         a_ready();
         acc_wait();                                                  // (all compute threads have arrived: nobody still reads k / v)
@@ -895,24 +483,14 @@ __global__ void __launch_bounds__(kThreads5, 1) vit_tc5_kernel(const Args a) {
   if (warp == kMmaWarp) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512) : "memory");
 }
 
-static size_t fixed_bytes5(int P, bool tca) {
+static size_t fixed_bytes5(int P) {
   const size_t PW = (size_t)P * kW;
-  return 1024 + (size_t)kPanels * kPanelBytes + (tca ? 0 : (size_t)kRows * kQStride * 4) + (size_t)2 * kCG * kRows * 4 + (6 + G_ROWS) * PW * 4 + 2 * PW * 4 + BAR_COUNT * 8 + 64;
+  return 1024 + (size_t)kPanels * kPanelBytes + (size_t)2 * kCG * kRows * 4 + (6 + G_ROWS) * PW * 4 + 2 * PW * 4 + BAR_COUNT * 8 + 64;
 }
-static int stages_for5(int P, bool tca) {
-  const long long left = 227LL * 1024 - (long long)fixed_bytes5(P, tca);
+static int stages_for5(int P) {
+  const long long left = 227LL * 1024 - (long long)fixed_bytes5(P);
   long long n = left / kChunkBytes;
   return (int)(n > kMaxStages ? kMaxStages : n);
-}
-// 0: the one-thread-per-row kernel above (CFPP_VIT_TC2_V1=1, A/B timing); 1: four threads per row, FP32 attention (CFPP_VIT_ATTN=fma; up to 64
-// tokens per sample: score table in operand panel 0); 2: four threads per row, attention on the tensor cores (default).  Read per call: the
-// tests compare the kernels in one process.
-static int tc5_mode(int n_tok) {
-  const char* e = getenv("CFPP_VIT_TC2_V1");
-  if (e && *e == '1') return 0;
-  const char* at = getenv("CFPP_VIT_ATTN");
-  if (at && at[0] == 'f') return n_tok <= 64 ? 1 : 0;
-  return 2;
 }
 
 }  // namespace vt2
@@ -921,7 +499,7 @@ using namespace cfpp;
 
 extern "C" int cfpp_vit_tc2_supported(int T, int patch_dim, int n_tok, int Cextra) {
   if (!(T >= 4 && T % 4 == 0 && T <= 192 && patch_dim >= 1 && patch_dim <= T && Cextra == 0 && n_tok >= 1 && n_tok <= vt2::kRows)) return 0;
-  return vt2::stages_for(T, (T + 63) / 64, (vt2::kRows / n_tok) * n_tok) >= 2 ? 1 : 0;
+  return vt2::stages_for5((T + 63) / 64) >= 2 ? 1 : 0;
 }
 
 /* chunks of the weight stream: embed (P x PD), then per layer qkv (3 x P), out (P x 1), mlp1 (P x P), mlp2 (P x P); P = ceil(T/64) */
@@ -937,27 +515,15 @@ extern "C" int cfpp_vit_tc2_fwd(const float* x, int64_t x_bstride, float* h, con
   CFPP_REQUIRE(d.n_tok == (d.H / d.p1) * (d.W / d.p2) && d.patch_dim == d.Cin * d.p1 * d.p2 && d.T % (d.p1 * d.p2) == 0, "vit_tc2: inconsistent descriptor");
   CFPP_REQUIRE((reinterpret_cast<uintptr_t>(wpack) & 15) == 0, "vit_tc2: wpack must be 16-byte aligned");
   if (B <= 0) return CFPP_OK;
-  vt2::Args a{x, x_bstride, h, d, (const uint8_t*)wpack, B, vt2::kRows / d.n_tok, 0, (d.T + 15) / 16 * 16, (d.T + 63) / 64, (d.patch_dim + 63) / 64, vt2::xs_of(d.T), 0, 0};
+  vt2::Args a{x, x_bstride, h, d, (const uint8_t*)wpack, B, vt2::kRows / d.n_tok, 0, (d.T + 15) / 16 * 16, (d.T + 63) / 64, (d.patch_dim + 63) / 64, 0};
   a.ntiles = (B + a.S - 1) / a.S;
-  a.xrows = a.S * d.n_tok;
-  if (const int mode5 = vt2::tc5_mode(d.n_tok)) {
-    const bool tca = mode5 == 2;
-    a.nstages = vt2::stages_for5(a.P, tca);
-    const size_t smem5 = vt2::fixed_bytes5(a.P, tca) + (size_t)a.nstages * vt2::kChunkBytes;
-    const int grid5 = a.ntiles < num_sms() ? a.ntiles : num_sms();
-#define CFPP_VT5(P_, T_) do { static DeviceHighWater attr5; \
-    if (attr5.raise((long long)smem5)) cudaFuncSetAttribute(vt2::vit_tc5_kernel<P_, T_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem5); \
-    vt2::vit_tc5_kernel<P_, T_><<<grid5, vt2::kThreads5, smem5, (cudaStream_t)stream>>>(a); } while (0)
-    if (tca) { if (a.P == 1) CFPP_VT5(1, true); else if (a.P == 2) CFPP_VT5(2, true); else CFPP_VT5(3, true); }
-    else { if (a.P == 1) CFPP_VT5(1, false); else if (a.P == 2) CFPP_VT5(2, false); else CFPP_VT5(3, false); }
-#undef CFPP_VT5
-    return check_launch("vit_cond_tc_fwd");
-  }
-  a.nstages = vt2::stages_for(d.T, a.P, a.xrows);
-  const size_t smem = vt2::fixed_bytes(d.T, a.P, a.xrows) + (size_t)a.nstages * vt2::kChunkBytes;
-  static DeviceHighWater attr;                                  // per device: one process may drive several GPUs
-  if (attr.raise((long long)smem)) cudaFuncSetAttribute(vt2::vit_tc2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  a.nstages = vt2::stages_for5(a.P);
+  const size_t smem = vt2::fixed_bytes5(a.P) + (size_t)a.nstages * vt2::kChunkBytes;
   const int grid = a.ntiles < num_sms() ? a.ntiles : num_sms();
-  vt2::vit_tc2_kernel<<<grid, vt2::kThreads, smem, (cudaStream_t)stream>>>(a);
+#define CFPP_VT5(P_) do { static DeviceHighWater attr;           /* per device: one process may drive several GPUs */ \
+    if (attr.raise((long long)smem)) cudaFuncSetAttribute(vt2::vit_tc5_kernel<P_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+    vt2::vit_tc5_kernel<P_><<<grid, vt2::kThreads5, smem, (cudaStream_t)stream>>>(a); } while (0)
+  if (a.P == 1) CFPP_VT5(1); else if (a.P == 2) CFPP_VT5(2); else CFPP_VT5(3);
+#undef CFPP_VT5
   return check_launch("vit_cond_tc_fwd");
 }

@@ -1,7 +1,6 @@
 """SimpleViT conditioner (reference layers/simple_vit.py:18-127): parameter container with the reference's module tree /
 state_dict names; forward is the fused CUDA kernel (cfpp_vit_cond_fwd)."""
 import ctypes
-import os
 
 import torch
 from torch import nn
@@ -109,7 +108,7 @@ class SimpleViT(nn.Module):
         g = self.geom
         lib = _cabi.lib()
         T, pd = g['T'], g['patch_dim']
-        small = bool(lib.cfpp_vit_tc_supported(T, pd, g['n_tok'], 0)) and os.environ.get('CFPP_VIT_GENERAL', '0') != '1'   # (=1: A/B the general kernel on the small shapes)
+        small = bool(lib.cfpp_vit_tc_supported(T, pd, g['n_tok'], 0))
         if not small and not lib.cfpp_vit_tc2_supported(T, pd, g['n_tok'], 0):
             return None
 
@@ -135,7 +134,7 @@ class SimpleViT(nn.Module):
         g = self.geom
         cextra = 0 if extra is None else extra.shape[1]
         cout = g['T'] // (g['p1'] * g['p2'])
-        if extra is None and img.is_cuda and ops.vit_tc_mode() != 'fma':
+        if extra is None and img.is_cuda:
             pk = self._tc_pack()
             if pk is not None:
                 return ops.vit_cond_tc(img, self.descriptor(g['Cin']), pk[0], cout, general=pk[1])

@@ -544,12 +544,6 @@ def vit_cond(x, desc: _cabi.VitDesc, cout, extra=None):
     return h
 
 
-def vit_tc_mode() -> str:
-    """'auto' (tensor cores whenever the shape has a plan) or 'fma' (force the FP32-FMA kernel) -- env CFPP_VIT."""
-    import os
-    return os.environ.get('CFPP_VIT', 'auto')
-
-
 def vit_tc_pack(mats):
     """mats: [(weight (out, in) row-major, n_rows, k_cols)] in chunk order -> packed fp16 hi/lo weight stream of cfpp_vit_tc_fwd."""
     _need_cuda(*[m[0] for m in mats])
@@ -699,7 +693,7 @@ def ctx_encode_batch(ctx, descs_dev, noises, widths, flow_width=0):
     cs = _carve(B, widths, ctx.device)
     arr = lambda ts: (vp * n)(*[vp(0 if t is None else t.data_ptr()) for t in ts])
     noises = [None if t is None else _f32(t) for t in noises]
-    if flow_width and os.environ.get('CFPP_ENC_FLOW', '1') != '0' and lib().cfpp_ctx_encode_flow_supported(int(flow_width)):
+    if flow_width and lib().cfpp_ctx_encode_flow_supported(int(flow_width)):
         _call('ctx_encode_batch_flow', (_p(ctx.contiguous()), _p(descs_dev), n, int(flow_width), arr(noises), arr(cs), arr(list(logp_all)), B, _stream()))
     else:
         _call('ctx_encode_batch', (_p(ctx.contiguous()), _p(descs_dev), n, arr(noises), arr(cs), arr(list(logp_all)), B, _stream()))

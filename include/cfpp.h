@@ -198,7 +198,7 @@ int cfpp_vit_tc_pack_chunk(const float* w, int ld, int n_rows, int k_cols, void*
 int cfpp_vit_tc_fwd(const float* x, int64_t x_bstride, float* h, const cfpp_vit_desc* desc, const void* wpack, int B, void* stream);
 
 /* General form (csrc/vit_tc2.cu): T <= 192 (T % 4 == 0), any token count up to 128 per sample, no concatenated context channels (the
- * ATM stack: T in {36, 72, 144, 152}).  Residual stream in shared memory, P = ceil(T/64) operand panels; the weight stream holds
+ * ATM stack: T in {36, 72, 144, 152}).  Four threads per token row, P = ceil(T/64) operand panels; the weight stream holds
  * cfpp_vit_tc2_chunks() chunks of the cfpp_vit_tc_pack_chunk format, one per (64-row output block n, 64-column input block p) of a
  * matrix, n outer / p inner, matrices in the order patch-embedding, then per layer to_qkv (192 x T), to_out (T x 64), mlp[1], mlp[3]. */
 int cfpp_vit_tc2_supported(int T, int patch_dim, int n_tok, int Cextra);

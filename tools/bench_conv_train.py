@@ -11,8 +11,8 @@ dev = 'cuda'
 
 REPS, WARM = int(os.environ.get('REPS', 10)), int(os.environ.get('WARM', 3))
 ONLY = os.environ.get('ONLY', '')              # e.g. ONLY=k3: the 3x3 shapes only
-VARIANTS = [v for v in os.environ.get('VARIANTS', 'new,nopf,old').split(',') if v]
-ENV = {'new': {}, 'nopf': {'CFPP_BWD_DATA3': '2'}, 'nt256': {'CFPP_BWD_DATA3': '3'}, 'old': {'CFPP_BWD_DATA3': '0', 'CFPP_CONV_ROWS': '0'}}
+VARIANTS = [v for v in os.environ.get('VARIANTS', 'new,old').split(',') if v]
+ENV = {'new': {}, 'old': {'CFPP_BWD_DATA3': '0', 'CFPP_CONV_ROWS': '0'}}
 
 
 def timeit(fn, n=REPS):
@@ -40,7 +40,7 @@ for cin, cout, H, W, K in SHAPES:
     for tag in VARIANTS:
         env = ENV[tag]
         os.environ.update(env)
-        if tag != 'nopf' and not ONLY:
+        if not ONLY:
             row[f'fwd_{tag}_us'] = round(timeit(lambda: ops.conv2d_fwd(x, cin, w, b, relu=True)), 1)
         row[f'bwd_data_{tag}_us'] = round(timeit(lambda: ops.conv2d_bwd_data(g, w, act=x)), 1)
         if tag == 'new' and not ONLY:

@@ -1,7 +1,6 @@
 #!/bin/bash
 mkdir -p gpurun_out
 timeout 300 python -m pytest tests/test_gpu_training.py -q -m gpu -k "conv2d_family" --timeout 120 > gpurun_out/r2bb_conv.log 2>&1; echo "conv tests rc=$?"; tail -2 gpurun_out/r2bb_conv.log
-ONLY=k3 VARIANTS=new,nt256,old timeout 300 python tools/bench_conv_train.py > gpurun_out/r2bb_conv_shapes.jsonl 2> gpurun_out/r2bb_conv_shapes.err; echo "shapes rc=$?"; cat gpurun_out/r2bb_conv_shapes.jsonl
 timeout 600 python tools/bench_training.py --workload cfg2 --batch 8192 --steps 5 --warmup 2 --graph > gpurun_out/r2bb_train_cfg2.json 2> gpurun_out/r2bb_train.err; echo "train rc=$?"
 python - <<P
 import json

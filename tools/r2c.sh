@@ -6,10 +6,9 @@ true
 B="python bench.py --steps 20 --warmup 5 --no-cpu-baseline --secondary="
 $B > gpurun_out/r2c_bench.json 2> gpurun_out/r2c_bench.err; echo "bench rc=$?"
 CFPP_C1X1_CTX=0 $B > gpurun_out/r2c_bench_noc1.json 2> gpurun_out/r2c_bench_noc1.err; echo "bench (two-kernel conv1x1) rc=$?"
-CFPP_ENC_FLOW=0 $B > gpurun_out/r2c_bench_noenc.json 2> gpurun_out/r2c_bench_noenc.err; echo "bench (per-sample encoder) rc=$?"
 python - <<'P'
 import json
-for f in ['r2c_bench','r2c_bench_noc1','r2c_bench_noenc']:
+for f in ['r2c_bench','r2c_bench_noc1']:
     try:
         d=json.loads(open(f'gpurun_out/{f}.json').read().strip().splitlines()[-1])
         print(f, round(d['value']), d['ms_per_step'], d['parity_at_bench_batch'].get('ok'))
