@@ -18,6 +18,8 @@
 // inner product stays at 3 instructions.  (Bucketing by scale context alone and carrying per-sample mean offsets in registers was
 // measured first: 4 instructions per evaluation plus an 8 x TM register reload per channel, 1.5-2.7x slower than this.)
 #include "common.cuh"
+#include "gmm_tc.cuh"
+#include <algorithm>
 
 namespace cfpp {
 namespace gt {
@@ -73,10 +75,10 @@ __global__ void prepare_kernel(const float* __restrict__ mG, const float* __rest
   }
 }
 
-// Single-CTA counting sort of the batch by scale context; buckets padded to whole tiles (perm = -1 in the padding).
+// Single-CTA counting sort of the batch by context tuple; buckets padded to whole tiles of ts samples (perm = -1 in the padding).
 // key = ctx[b,0] (one feature) or ctx[b,0] * card1 + ctx[b,1] (two features)
 __global__ void __launch_bounds__(1024) bucket_kernel(const int64_t* __restrict__ ctx, int n_ctx, int card1, int B, int NB,
-                                                      int* __restrict__ perm, int* __restrict__ tile_vs, int* __restrict__ n_tiles) {
+                                                      int ts, int* __restrict__ perm, int* __restrict__ tile_vs, int* __restrict__ n_tiles) {
   extern __shared__ int sh[];
   int* cnt = sh; int* base = sh + NB; int* cur = sh + 2 * NB;
   __shared__ int total_tiles;
@@ -91,24 +93,26 @@ __global__ void __launch_bounds__(1024) bucket_kernel(const int64_t* __restrict_
   __syncthreads();
   if (threadIdx.x == 0) {
     int t = 0;
-    for (int k = 0; k < NB; ++k) { base[k] = t; t += (cnt[k] + TS - 1) / TS; }
+    for (int k = 0; k < NB; ++k) { base[k] = t; t += (cnt[k] + ts - 1) / ts; }
     total_tiles = t; *n_tiles = t;
   }
   __syncthreads();
   for (int k = threadIdx.x; k < NB; k += blockDim.x) {
-    const int nt = (cnt[k] + TS - 1) / TS;
+    const int nt = (cnt[k] + ts - 1) / ts;
     for (int t = 0; t < nt; ++t) tile_vs[base[k] + t] = k;
   }
-  for (int i = threadIdx.x; i < total_tiles * TS; i += blockDim.x) perm[i] = -1;
+  for (int i = threadIdx.x; i < total_tiles * ts; i += blockDim.x) perm[i] = -1;
   __syncthreads();
   // stable within a bucket is not required for the result; atomics give an arbitrary but valid order
-  for (int b = threadIdx.x; b < B; b += blockDim.x) { const int k = key_of(b); perm[base[k] * TS + atomicAdd(&cur[k], 1)] = b; }
+  for (int b = threadIdx.x; b < B; b += blockDim.x) { const int k = key_of(b); perm[base[k] * ts + atomicAdd(&cur[k], 1)] = b; }
 }
 
 struct Args {
   const float* x; int64_t x_bstride;
   const float2* PT; const float* LB;
   const int* perm; const int* tile_vs; const int* n_tiles;      // NULL: identity order, no context, grid.x tiles; tile_vs holds the tile's context key
+  int tile_shift;                                               // buckets hold whole tiles of TS << tile_shift samples (n_tiles, tile_vs count those)
+  const int* flags; int ftiles;                                 // non-NULL: tile_kernel only recomputes the slices that gmm_tc flagged ([nsplit][ftiles])
   int key_div, scale_in_low;                                    // key -> (mean context, scale context): two features: (key / key_div, key % key_div); one: (key, key)
   const float* mtab; int mwidth, moff;                          // mean offsets of a tile: mtab + mean_ctx * mwidth + moff + mk * D + d
   float* part;                                                  // [nsplit][slots][MKP]
@@ -129,7 +133,8 @@ template <int TM, bool OFF>
 __global__ void __launch_bounds__(256, 2) tile_kernel(const Args a) {     // <= 128 registers: three 160-thread CTAs per SM at M*K = 80
   extern __shared__ float4 gt_smem4[];
   const int tile = blockIdx.x, split = blockIdx.y;
-  if (a.n_tiles && tile >= *a.n_tiles) return;
+  if (a.n_tiles && (tile >> a.tile_shift) >= *a.n_tiles) return;
+  if (a.flags && !a.flags[(int64_t)split * a.ftiles + (tile >> a.tile_shift)]) return;
   const int MKP = a.MKP;
   float* xs = reinterpret_cast<float*>(gt_smem4);                 // [2][TS][XS]
   float2* ps = reinterpret_cast<float2*>(xs + 2 * TS * XS);       // [2][EC][MKP]
@@ -140,7 +145,7 @@ __global__ void __launch_bounds__(256, 2) tile_kernel(const Args a) {     // <= 
     bidx[i] = a.perm ? a.perm[slot] : (slot < a.B ? slot : -1);
   }
   __syncthreads();
-  const int key = a.tile_vs ? a.tile_vs[tile] : 0;
+  const int key = a.tile_vs ? a.tile_vs[tile >> a.tile_shift] : 0;
   const int vs = a.scale_in_low ? key % a.key_div : key, vm = a.scale_in_low ? key / a.key_div : key;
   const float2* PTv = a.PT + (int64_t)vs * a.EP * MKP;
   const int e_begin = split * a.esplit, e_end = min(a.E, e_begin + a.esplit);
@@ -249,10 +254,11 @@ __global__ void finish_kernel(const Args a) {
   const int64_t total = (int64_t)a.slots * a.M;
   for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < total; idx += (int64_t)gridDim.x * blockDim.x) {
     const int slot = (int)(idx / a.M), m = (int)(idx - (int64_t)slot * a.M);
-    if (a.n_tiles && slot >= *a.n_tiles * TS) continue;
+    const int ts = TS << a.tile_shift;
+    if (a.n_tiles && slot >= *a.n_tiles * ts) continue;
     const int b = a.perm ? a.perm[slot] : (slot < a.B ? slot : -1);
     if (b < 0) continue;
-    const int key = a.tile_vs ? a.tile_vs[slot / TS] : 0;
+    const int key = a.tile_vs ? a.tile_vs[slot / ts] : 0;
     const int vs = a.scale_in_low ? key % a.key_div : key;
     float c[64];
     float mx = -INFINITY;
@@ -272,7 +278,7 @@ static inline int64_t align_up(int64_t v, int64_t al) { return (v + al - 1) / al
 static inline int mkp_of(int MK) { return (MK + 3) & ~3; }
 static inline int ep_of(int E) { return (E + EC - 1) / EC * EC; }
 static inline int tm_of(int MKP) { return MKP >= 64 ? 4 : (MKP >= 32 ? 2 : 1); }      // threads = 8 * MKP / TM <= 256
-static inline int64_t max_tiles(int B, int n_keys) { return ((int64_t)B + TS - 1) / TS + (n_keys > 1 ? n_keys : 0); }
+static inline int64_t max_tiles(int B, int n_keys, int ts = TS) { return ((int64_t)B + ts - 1) / ts + (n_keys > 1 ? n_keys : 0); }
 // Slices of e per tile: enough CTAs for ~4 rounds of the ~3 CTAs an SM holds (a 1.05-wave grid runs at half speed), counted on the
 // expected number of non-empty tiles (buckets are padded by half a tile on average; the launch grid covers the worst case).
 static inline int splits_for(int B, int n_keys, int E) {
@@ -306,14 +312,30 @@ extern "C" int cfpp_gmm_tile_prepare(const float* mG, const float* sG, const flo
   return check_launch("gmm_tile_prepare");
 }
 
-extern "C" int64_t cfpp_gmm_tile_workspace_bytes(int B, int M, int K, int D, int HW, int n_keys) {
-  if (n_keys < 1 || n_keys > 4096) return -1;
-  const int MKP = gt::mkp_of(M * K);
-  const int64_t tiles = gt::max_tiles(B, n_keys);
-  const int nsplit = gt::splits_for(B, n_keys, D * HW);
-  return gt::align_up((int64_t)nsplit * tiles * gt::TS * MKP * 4, 256) + gt::align_up(tiles * gt::TS * 4, 256) + gt::align_up(tiles * 4, 256) + 256;
+// Workspace: partial sums, bucket permutation, tile keys, tile count and the tensor-core kernel's guard flags, sized for the larger of
+// the two geometries (64-sample tiles of tile_kernel, 128-sample tiles of gmm_tc).
+struct Workspace { int64_t part, perm, tile_vs, flags; };
+static Workspace ws_layout(int B, int M, int K, int D, int HW, int n_keys) {
+  const int MKP = gt::mkp_of(M * K), E = D * HW;
+  const int64_t t64 = gt::max_tiles(B, n_keys), t128 = gt::max_tiles(B, n_keys, gtc::TS);
+  const int64_t ns64 = gt::splits_for(B, n_keys, E), ns128 = gtc::splits_for(B, n_keys, E, M * K);
+  Workspace w;
+  w.part = gt::align_up(std::max(ns64 * t64 * gt::TS, ns128 * t128 * gtc::TS) * MKP * 4, 256);
+  w.perm = gt::align_up(std::max(t64 * gt::TS, t128 * gtc::TS) * 4, 256);
+  w.tile_vs = gt::align_up(std::max(t64, t128) * 4, 256);
+  w.flags = gt::align_up(ns128 * t128 * 4, 256);
+  return w;
 }
 
+extern "C" int64_t cfpp_gmm_tile_workspace_bytes(int B, int M, int K, int D, int HW, int n_keys) {
+  if (n_keys < 1 || n_keys > 4096) return -1;
+  const Workspace w = ws_layout(B, M, K, D, HW, n_keys);
+  return w.part + w.perm + w.tile_vs + 256 + w.flags;
+}
+
+// Tensor-core path (gmm_tc.cu) when x rows can be read as 16-byte vectors and M*K > 48; the exact tile_kernel otherwise, and for every
+// slice whose accuracy guard gmm_tc flags.  tile_kernel spends 3 M*K FP32 instructions per element of x, gmm_tc a fixed conversion of x
+// into operands: on one B200 the tensor cores win at M*K = 80 (cfg2: 0.66 -> 0.42 ms per step) and lose at M*K = 8 (cfg4: 0.065 -> 0.085 ms).
 extern "C" int cfpp_gmm_tile_logprob(const float* x, int64_t x_bstride, const void* table, const int64_t* ctx, int n_ctx,
                                      const int* cards, const float* mean_table, int mean_width, int mean_off,
                                      const float* logp_c, float logp_scale, float* out, void* workspace,
@@ -329,33 +351,51 @@ extern "C" int cfpp_gmm_tile_logprob(const float* x, int64_t x_bstride, const vo
   if (B <= 0) return CFPP_OK;
   cudaStream_t st = (cudaStream_t)stream;
   const int MK = M * K, MKP = gt::mkp_of(MK), E = D * HW, EP = gt::ep_of(E);
-  const int64_t tiles = gt::max_tiles(B, n_keys);
-  const int nsplit = gt::splits_for(B, n_keys, E);
+  const bool tc = MK > 48 && ((reinterpret_cast<uintptr_t>(x) & 15) == 0) && (x_bstride % 4 == 0) && (E % 4 == 0);
+  const int ts = tc ? gtc::TS : gt::TS;
+  const int64_t tiles = gt::max_tiles(B, n_keys, ts);
+  const int nsplit = tc ? gtc::splits_for(B, n_keys, E, MK) : gt::splits_for(B, n_keys, E);
   const int nch = EP / gt::EC, per = (nch + nsplit - 1) / nsplit;
   gt::Args a{};
   a.x = x; a.x_bstride = x_bstride;
   a.PT = (const float2*)table;
   a.LB = (const float*)((const char*)table + gt::align_up((int64_t)n_scale_ctx * EP * MKP * 8, 256));
+  const Workspace w = ws_layout(B, M, K, D, HW, n_keys);
   char* p = (char*)workspace;
-  a.part = (float*)p; p += gt::align_up((int64_t)nsplit * tiles * gt::TS * MKP * 4, 256);
-  int* perm = (int*)p; p += gt::align_up(tiles * gt::TS * 4, 256);
-  int* tile_vs = (int*)p; p += gt::align_up(tiles * 4, 256);
-  int* n_tiles = (int*)p;
+  a.part = (float*)p; p += w.part;
+  int* perm = (int*)p; p += w.perm;
+  int* tile_vs = (int*)p; p += w.tile_vs;
+  int* n_tiles = (int*)p; p += 256;
+  int* flags = (int*)p;
   a.key_div = n_ctx == 2 ? cards[1] : 1; a.scale_in_low = n_ctx == 2 ? 1 : 0;
   a.mtab = mean_table; a.mwidth = mean_width; a.moff = mean_off;
   a.logp_c = logp_c; a.logp_scale = logp_scale; a.out = out;
   a.B = B; a.M = M; a.K = K; a.MK = MK; a.MKP = MKP; a.D = D; a.HW = HW; a.E = E; a.EP = EP;
-  a.esplit = per * gt::EC; a.nsplit = nsplit; a.slots = (int)(tiles * gt::TS);
+  a.esplit = per * gt::EC; a.nsplit = nsplit; a.slots = (int)(tiles * ts);
+  a.tile_shift = tc ? 1 : 0;
   if (n_ctx > 0) {
-    gt::bucket_kernel<<<1, 1024, 3 * n_keys * sizeof(int), st>>>(ctx, n_ctx, n_ctx == 2 ? cards[1] : 1, B, n_keys, perm, tile_vs, n_tiles);
+    gt::bucket_kernel<<<1, 1024, 3 * n_keys * sizeof(int), st>>>(ctx, n_ctx, n_ctx == 2 ? cards[1] : 1, B, n_keys, ts, perm, tile_vs, n_tiles);
     int rc = check_launch("gmm_tile_bucket");
     if (rc) return rc;
     a.perm = perm; a.tile_vs = tile_vs; a.n_tiles = n_tiles;
   }
+  if (tc) {
+    gtc::Args g{};
+    g.x = x; g.x_bstride = x_bstride; g.PT = a.PT; g.LB = a.LB;
+    g.perm = a.perm; g.tile_vs = a.tile_vs; g.n_tiles = a.n_tiles;
+    g.key_div = a.key_div; g.scale_in_low = a.scale_in_low;
+    g.mtab = mean_table; g.mwidth = mean_width; g.moff = mean_off;
+    g.part = a.part; g.flags = flags; g.has_logp = logp_c != nullptr;
+    g.B = B; g.K = K; g.MK = MK; g.MKP = MKP; g.N = gtc::n_of(MK); g.D = D; g.HW = HW; g.E = E; g.EP = EP;
+    g.esplit = a.esplit; g.nsplit = nsplit; g.slots = a.slots; g.tiles = (int)tiles;
+    int rc = gtc::launch(g, st);
+    if (rc) return rc;
+    a.flags = flags; a.ftiles = (int)tiles;
+  }
   const int TM = gt::tm_of(MKP);
   const int threads = gt::SGS * (MKP / TM);
   const size_t smem = (size_t)2 * gt::TS * gt::XS * 4 + (size_t)2 * gt::EC * MKP * 8;
-  dim3 grid((unsigned)tiles, nsplit);
+  dim3 grid((unsigned)(tiles << a.tile_shift), nsplit);
   const bool offs = mean_table != nullptr;
 #define CFPP_GT_LAUNCH(TMV, OFFV)                                                                                          \
   do {                                                                                                                     \

@@ -244,7 +244,10 @@ int64_t cfpp_gmm_ctxtab_workspace_bytes(int B, int M, int K, int D, int HW, int 
  *                           scale contexts) and one mean-offset row mean_table[ctx[b,0]][mean_off + (m*K+k)*D + d] (mean_table NULL: none).
  * For ContextEncoder(contexts,'embed','eyesample') ('b (p m k d)', model.py:157,162): n_ctx == 2 -> means = tables[0], scales = tables[1],
  * offsets 0; n_ctx == 1 -> both from tables[0]: mean_off 0, scale_off M*K*D.  n_keys = product of cards (<= 4096).
- * M*K <= 128 (padded to a multiple of 4), K <= 64.  *_bytes return -1 when unsupported. */
+ * M*K <= 128 (padded to a multiple of 4), K <= 64.  *_bytes return -1 when unsupported.
+ * When M*K > 48 and x rows can be read as 16-byte vectors (x, x_bstride 16-byte aligned, D*HW a multiple of 4), cfpp_gmm_tile_logprob evaluates
+ * the density on the tensor cores (csrc/gmm_tc.cu: tiles of 128 samples, tf32 hi/lo operands, K = 2 D*HW); a slice of a tile whose
+ * parameters fail that kernel's accuracy guard, and every other x, takes the register-tiled kernel.  Both are deterministic. */
 int64_t cfpp_gmm_tile_table_bytes(int M, int K, int D, int HW, int n_scale_ctx);
 int cfpp_gmm_tile_prepare(const float* mG, const float* sG, const float* wG, const float* scale_table, int scale_width,
                           int scale_off, int n_scale_ctx, void* table, int M, int K, int D, int HW, void* stream);
