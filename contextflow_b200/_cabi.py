@@ -52,6 +52,9 @@ _SIGNATURES = {
     'cfpp_student_table_floats': (i64, [i32, i32, i32]),
     'cfpp_student_prep': (i32, [vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp]),
     'cfpp_student_logprob': (i32, [vp, vp, vp, i32, i32, i32, i32, vp]),
+    'cfpp_student_train_fwd': (i32, [vp, i64, vp, vp, vp, i32, i32, i32, i32, vp]),
+    'cfpp_student_train_bwd_workspace_floats': (i64, [i32, i32, i32, i32]),
+    'cfpp_student_train_bwd': (i32, [vp, i64, vp, vp, vp, vp, vp, vp, vp, vp, i64, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp]),
     'cfpp_bias_rows_relu': (i32, [vp, vp, i32, i32, i32, vp]),
     'cfpp_gmm_ctx_param_bwd': (i32, [vp, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]),
     'cfpp_squeeze_fwd': (i32, [vp, vp, i32, i32, i32, i32, i32, i32, vp]),

@@ -1,9 +1,11 @@
 """StudentMixtureDistribution (reference layers/distributions/student.py:44-111, `--dist tdist`).  create_model cannot build it
-(model.py:163 passes `components=`, which student.py:44 rejects), but the class can be constructed directly; log_prob runs the CUDA kernel."""
+(model.py:163 passes `components=`, which student.py:44 rejects), but the class can be constructed directly.  log_prob runs CUDA kernels:
+for scoring, and under autograd (training.StudentMixtureFn) with gradients for mG, sG, wG, mS, sS, wS and for the input, so the prior
+trains as FlowSequential.dist or inside a SplitPrior.  vS stays frozen, as in the reference (student.py:59)."""
 import torch
 import torch.nn as nn
 
-from ... import ops
+from ... import ops, training
 from ..flowlayer import PackCache, inference_only
 
 __all__ = ['StudentMixtureDistribution']
@@ -36,6 +38,9 @@ class StudentMixtureDistribution(nn.Module):
         return self.log_prob(input, context)
 
     def log_prob(self, input, context=None):
+        if training.wants_grad(input, self.mG, self.sG, self.wG, self.mS, self.sS, self.wS):
+            inference_only(self.vS)
+            return training.StudentMixtureFn.apply(input, self, 0, self.mG, self.sG, self.wG, self.mS, self.sS, self.wS)
         src = [self.mG, self.sG, self.wG, self.mS, self.sS, self.wS, self.vS]
         for p in src:
             inference_only(p)

@@ -1,7 +1,7 @@
 """SplitPrior: factor out the second half of the channels under a (context-conditioned) mixture prior
 (reference layers/splitprior.py:7-15)."""
 from .. import ops, training
-from .flowlayer import FlowLayer
+from .flowlayer import FlowLayer, inference_only
 
 
 class SplitPrior(FlowLayer):
@@ -11,6 +11,9 @@ class SplitPrior(FlowLayer):
 
     def forward(self, x, context=None):
         d = self.dist
+        if hasattr(d, 'mS') and training.wants_grad(x, d.mG, d.sG, d.wG, d.mS, d.sS, d.wS):     # Student-t mixture: it has an mG too
+            inference_only(d.vS)                                    # the degrees of freedom have no backward kernel (frozen in the reference)
+            return training.StudentMixtureFn.apply(x, d, x.shape[1] // 2, d.mG, d.sG, d.wG, d.mS, d.sS, d.wS)
         if not getattr(d, 'context_net', None) and hasattr(d, 'mG') and training.wants_grad(x, d.mG, d.sG, d.wG):
             return training.SplitPriorFn.apply(x, d.mG, d.sG, d.wG, d)
         if getattr(d, 'context_net', None) and hasattr(d, 'mG') and training.wants_grad(x, *d.context_net.parameters()):

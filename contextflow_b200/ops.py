@@ -1232,6 +1232,46 @@ def student_logprob(x, table, M, K):
     return logp
 
 
+def student_train_fwd(x, table, M, K):
+    """student_logprob under autograd: also the responsibilities resp (B, M, 2, K) of the Gaussian (0) and Student-t (1) components.
+    x (B, D, H, W) may be a channel slice of a contiguous tensor (SplitPrior)."""
+    _need_cuda(x, table)
+    xv, bstride = _half_view(x)
+    B = x.shape[0]
+    n = x[0].numel() if B else 1
+    logp = torch.empty((B, M), device=x.device, dtype=torch.float32)
+    resp = torch.empty((B, M, 2, K), device=x.device, dtype=torch.float32)
+    _set_work(bytes=4.0 * B * n + 4.0 * B * M * (1 + 2 * K), flops=12.0 * B * M * K * n)
+    _call('student_train_fwd', (_p(xv), bstride, _p(table), _p(logp), _p(resp), B, M, K, n, _stream()))
+    return logp, resp
+
+
+def student_train_bwd(x, table, sG, wG, sS, wS, resp, g, need_dx=True, need_params=True, dx_out=None):
+    """-> dx, (dmG, dsG, dwG, dmS, dsS, dwS) or None.  dx_out: optional (B, D, H, W) channel-slice view of a wider contiguous tensor that
+    receives dx in place."""
+    _need_cuda(x, table, g); g = _f32(g)
+    xv, bstride = _half_view(x)
+    B = x.shape[0]
+    M, K = resp.shape[1], resp.shape[3]
+    n = x[0].numel()
+    if dx_out is not None:
+        dv, dstride = _half_view(dx_out)
+        assert dv.data_ptr() == dx_out.data_ptr(), 'student_train_bwd: dx_out must be a channel slice of a contiguous tensor'
+        dx = dx_out
+    else:
+        dstride = n
+        dx = torch.empty((B,) + tuple(x.shape[1:]), device=x.device, dtype=torch.float32) if need_dx else None
+    grads = None
+    if need_params:
+        grads = tuple(torch.empty(p.shape, device=x.device, dtype=torch.float32) for p in (sG, sG, wG, sS, sS, wS))
+    ws = torch.empty(int(lib().cfpp_student_train_bwd_workspace_floats(B, M, K, n)), device=x.device, dtype=torch.float32)
+    _set_work(bytes=4.0 * B * n * ((2 if need_dx else 0) + (1 if need_params else 0)), flops=(24.0 if need_params else 12.0) * B * M * K * n)
+    gp = [None] * 6 if grads is None else [_p(t) for t in grads]
+    _call('student_train_bwd', (_p(xv), bstride, _p(table), _p(_f32(sG)), _p(_f32(wG)), _p(_f32(sS)), _p(_f32(wS)), _p(_f32(resp)), _p(g),
+                                _p(dx), dstride, *gp, _p(ws), B, M, K, n, _stream()))
+    return dx, grads
+
+
 def bias_rows_relu_(a, bias):
     """a (B, C, H, W) <- relu(a + bias[b, c]) in place (conventional coupling's first convolution, coupling.py:47)."""
     _need_cuda(a, bias)

@@ -221,6 +221,42 @@ class SplitPriorFn(Function):
         return dx, dmG, dsG, dwG, None
 
 
+class StudentMixtureFn(Function):
+    """StudentMixtureDistribution.log_prob (student.py:76-98); the degrees of freedom vS stay frozen, as in the reference (student.py:59).
+    `split` > 0: the SplitPrior form -- x is the full tensor, the mixture scores x[:, split:] and the Function also returns x[:, :split]
+    (splitprior.py:12-15)."""
+
+    @staticmethod
+    def forward(ctx, x, dist, split, mG, sG, wG, mS, sS, wS):
+        src = [mG, sG, wG, mS, sS, wS, dist.vS]
+        table = dist._tables.get('student', src, lambda: ops.student_table(*[p.detach() for p in src]))
+        logp, resp = ops.student_train_fwd(x[:, split:] if split else x, table, dist.M, dist.K)
+        ctx.save_for_backward(x, table, resp, sG, wG, sS, wS)
+        ctx.M, ctx.split = dist.M, split
+        if split:
+            return ops.slice_channels(x, 0, split), logp
+        return logp
+
+    @staticmethod
+    def backward(ctx, *grads):
+        x, table, resp, sG, wG, sS, wS = ctx.saved_tensors
+        split = ctx.split
+        dx0, g = grads if split else (None, grads[0])
+        g = torch.zeros((x.shape[0], ctx.M), device=x.device) if g is None else g.contiguous()
+        need_dx = ctx.needs_input_grad[0]
+        need_params = any(ctx.needs_input_grad[3:])
+        dx = None
+        if split and need_dx:
+            dx = torch.empty_like(x)
+            ops.place_channels(_zeros_like_if_none(dx0, (x.shape[0], split) + tuple(x.shape[2:]), x.device).contiguous(), dx, 0)
+        dxs, pg = ops.student_train_bwd(x[:, split:] if split else x, table, sG.detach(), wG.detach(), sS.detach(), wS.detach(), resp, g,
+                                        need_dx=need_dx, need_params=need_params, dx_out=dx[:, split:] if dx is not None else None)
+        if not split:
+            dx = dxs
+        pg = pg if pg is not None else (None,) * 6
+        return (dx, None, None, *[d if need else None for d, need in zip(pg, ctx.needs_input_grad[3:])])
+
+
 class LdjSumFn(Function):
     """logprob + ((0 + ldj_0) + ldj_1) + ...  (flowsequential.py:20-27); a (B,) / (B,1) term receives the row sum of the gradient."""
 

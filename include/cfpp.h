@@ -511,6 +511,16 @@ int64_t cfpp_student_table_floats(int M, int K, int n);
 int cfpp_student_prep(const float* mG, const float* sG, const float* wG, const float* mS, const float* sS, const float* wS,
                       const float* vS, float* table, int M, int K, int n, void* stream);
 int cfpp_student_logprob(const float* x, const float* table, float* logp, int B, int M, int K, int n, void* stream);
+/* Training direction (vS frozen, as in the reference).  train_fwd: logp as above and resp (B, M, 2, K) = softmax_k of the Gaussian (0)
+ * and Student-t (1) component terms, x rows at x_bstride floats.  train_bwd: from g (B, M) = dL/dlogp, dx (rows at dx_bstride; NULL
+ * skips it) and, unless dmG is NULL, dmG, dsG, dmS, dsS (M, K, n) and dwG, dwS (M, K).  sG, wG, sS, wS are the raw parameters; table is
+ * the one train_fwd read.  M*K <= 768.  Parameter sums run over fixed chunks of samples, then in chunk order: no atomics. */
+int cfpp_student_train_fwd(const float* x, int64_t x_bstride, const float* table, float* logp, float* resp, int B, int M, int K, int n,
+                           void* stream);
+int64_t cfpp_student_train_bwd_workspace_floats(int B, int M, int K, int n);
+int cfpp_student_train_bwd(const float* x, int64_t x_bstride, const float* table, const float* sG, const float* wG, const float* sS,
+                           const float* wS, const float* resp, const float* g, float* dx, int64_t dx_bstride, float* dmG, float* dsG,
+                           float* dwG, float* dmS, float* dsS, float* dwS, float* workspace, int B, int M, int K, int n, void* stream);
 /* Training of the conventional (concatenated-context, contextflow = False) specialists.
  * bias_rows_relu: a (B, C, HW) <- relu(a + bias[b, c]) in place: conv1 of coupling.py:47 = W1[:, :D] x0 + (b1 + W1[:, D:] CN(c)).
  * gmm_ctx_param_bwd: gradients of the mixture's own mG, sG (M, K, D, HW) and wG (M, K) when they train beside the context offsets c
